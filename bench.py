@@ -15,8 +15,10 @@ Further top-level keys of the same JSON line (each with its own roofline / e2e /
   `co_occurrence`           — configs[3]: 500 000 points, 20 clusters, 49 radii, through `sq.gr.co_occurrence`;
   `ripley_L`                — configs[4]: 300 000 cells, 12 clusters, through `sq.gr.ripley(mode="L")`.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--skip-moran] [--skip-pairs] [--skip-cpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--skip-moran] [--skip-pairs] [--skip-cpu] [--dump-outputs DIR]
 N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+--dump-outputs DIR writes what the timed calls returned in their last step (rank 0) as DIR/<name>.npy, float64, so that two
+builds can be compared output for output: every input is generated from fixed seeds.
 """
 
 from __future__ import annotations
@@ -44,6 +46,26 @@ CONFIG = {"workload": WORKLOAD, "n_perms_per_gpu": CFG2["n_perms"], "rng": "nump
 # warp instructions per evaluated unordered pair of the tiled pair kernel (profiles/r01_prof_cooc_metrics.csv:
 # smsp__inst_executed.sum = 2.448e10 for 200 000 points = 2.0e10 pair evaluations) and the issue peak they are held against
 PAIR_WARP_INSTR = 2.448e10 / (200_000 * 199_999 / 2)
+# --dump-outputs: name -> what the timed calls returned in their last step; an array larger than DUMP_ARRAY_BYTES is stored as a
+# fixed, seeded sample of its rows (plus `<name>_rows`, the row indices), which keeps a dump under DUMP_TOTAL_BYTES
+OUTPUTS: dict[str, np.ndarray] = {}
+DUMP_ARRAY_BYTES, DUMP_TOTAL_BYTES = 8 << 20, 64 << 20
+
+
+def dump_outputs(path: str) -> None:
+    os.makedirs(path, exist_ok=True)
+    arrays = {}
+    for name, a in OUTPUTS.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            keep = max(1, DUMP_ARRAY_BYTES // (a.nbytes // a.shape[0]))
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))
+            a, arrays[f"{name}_rows"] = a[rows], rows.astype(np.float64)
+        arrays[name] = a
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_TOTAL_BYTES, f"--dump-outputs would write {total} bytes"
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def _peaks():
@@ -293,8 +315,9 @@ def run_reference(args, rank, ws):
     t_all = time.perf_counter()
     for k in range(args.steps):
         t0 = time.perf_counter()
-        ref.nhood_perm_counts(g.indptr, g.indices, base, CFG2["n_cls"], spawn_states(k, p_s), n_threads=cores)
+        counts = ref.nhood_perm_counts(g.indptr, g.indices, base, CFG2["n_cls"], spawn_states(k, p_s), n_threads=cores)
         rates.append(p_s / (time.perf_counter() - t0))
+    OUTPUTS["nhood_counts"] = counts
     dt = time.perf_counter() - t_all
     val = args.steps * p_s / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "permutations/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -306,6 +329,8 @@ def run_reference(args, rank, ws):
                              "serial_value": serial},
             "e2e": {"value": val, "unit": "permutations/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs)
 
 
 def _fit_extrapolate(ns, secs, n_target):
@@ -353,6 +378,7 @@ def bench_moran(ctx, rank, ws, steps, warmup, flush, skip_cpu):
     ms = _timed_steps(lambda: plan.run_async("moran"), steps, flush, ws)
     launches = (ctx.launches - l0) // max(steps, 1)
     score = plan.download()
+    OUTPUTS["moran_I"] = score
     nnz_x = int(np.diff(x.indptr).sum()) if ws == 1 else int(x.nnz * (hi - lo) / G)
     algo_bytes = 8 * x.nnz + 8 * (G + 1) + 8 * g.nnz + 4 * (n + 1) + 8 * G  # whole call, SURVEY 8(d)
     peak, _, _ = _peaks()
@@ -417,6 +443,7 @@ def bench_cooc(ctx, rank, ws, skip_cpu):
         occ, iv = sq.gr.co_occurrence(ad, "cluster", copy=True)
         _barrier_sync(ws)
         reps.append(_max_over_ranks(time.perf_counter() - t0, ws))
+    OUTPUTS["cooc_occ"], OUTPUTS["cooc_interval"] = occ, iv
     ctx.profile(True)
     ctx.profile_reset()
     sq.gr.co_occurrence(ad, "cluster", copy=True)
@@ -477,6 +504,8 @@ def bench_ripley(ctx, rank, ws, skip_cpu):
         res = sq.gr.ripley(ad, "cluster", **kw)
         _barrier_sync(ws)
         reps.append(_max_over_ranks(time.perf_counter() - t0, ws))
+    OUTPUTS.update(ripley_L_stat=res["L_stat"]["stats"].to_numpy(), ripley_sims_stat=res["sims_stat"]["stats"].to_numpy(), ripley_bins=res["bins"],
+                   ripley_pvalues=res["pvalues"])
     ctx.profile(True)
     ctx.profile_reset()
     sq.gr.ripley(ad, "cluster", **kw)
@@ -529,7 +558,10 @@ def main():
     ap.add_argument("--perms", type=int, default=CFG2["n_perms"])
     ap.add_argument("--shuffle-threads", type=int, default=0)
     ap.add_argument("--shuffle-algo", type=int, default=-1)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed calls returned in their last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
 
     if args.impl == "reference":
@@ -594,6 +626,8 @@ def main():
             m, s = last["mean"].ravel(), last["std"].ravel()
         counts = plan.download()
         assert (counts.reshape(P, -1).sum(axis=1, dtype=np.int64) == g.nnz).all(), "count checksum failed"
+        tag = "nhood_fast" if fast else "nhood"
+        OUTPUTS.update({f"{tag}_counts": counts, f"{tag}_mean": m.reshape(n_cls, n_cls), f"{tag}_std": s.reshape(n_cls, n_cls)})
         # per-kernel-class CUDA-event times of ONE step (launches synchronised, not part of the timed region)
         ctx.profile(True)
         ctx.profile_reset()
@@ -656,6 +690,7 @@ def main():
         return _max_over_ranks((time.perf_counter() - t0) / e2e_steps, ws), res
 
     t_e2e, res = time_api("numpy")
+    OUTPUTS["nhood_zscore"] = res.zscore
     h2d = int(g.indptr.nbytes + g.indices.nbytes + 2 * base.nbytes + states.nbytes)
     d2h = int(3 * n_cls * n_cls * 8)  # observed counts + mean + std (the per-permutation counts stay on the device)
     e2e = {"value": ws * P / t_e2e, "unit": "permutations/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "seconds_per_call": t_e2e,
@@ -695,6 +730,8 @@ def main():
         stat5 = torch.empty((2, 144), dtype=torch.float64, device="cuda")
         step5()
         ms5 = _timed_steps(step5, max(1, min(args.steps, 3)), flush, ws)
+        if ws == 1:
+            OUTPUTS["nhood_cfg5_mean"], OUTPUTS["nhood_cfg5_std"] = stat5.cpu().numpy().reshape(2, 12, 12)
         cfg5 = {"metric": "nhood_enrichment permutations/s (configs[4]: 300k cells, 12 clusters, kNN k=6 directed graph, n_perms=10000 in total)",
                 "value": P5 / (ms5 / 1e3), "unit": "permutations/s", "ms_per_step": ms5, "scaling": "strong", "perms_per_rank": hi5 - lo5,
                 "graph_build_seconds": t_graph, "nnz": int(adj5.nnz),
@@ -735,6 +772,8 @@ def main():
                 "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline, "cpu_baseline": cpu,
                 "fast": fast, "roofline_fast": roofline_fast, "nhood_cfg5_strong": cfg5, "moran": moran, "co_occurrence": cooc, "ripley_L": rip}
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs)
     plan.close()
     if ws > 1:
         import torch.distributed as dist

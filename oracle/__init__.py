@@ -10,9 +10,9 @@ Contents
   function cites the reference ``file:line`` it follows.
 * ``ref.py`` — numpy-level wrappers around the C library plus the float/host post-processing of each
   reference function (z-scores, occ ratio, L estimate, analytic p-values) restated in numpy.
-* ``_refload.py`` — stub-import loader that runs the UNMODIFIED reference modules from ``/root/reference`` in
-  the build container; used to pin the restatement (``tests/test_oracle_vs_reference.py``) and to generate
-  ``tests/golden/*.npz`` (``tests/golden/make_golden.py``).
+* ``_refload.py`` — stub-import loader that runs the UNMODIFIED reference modules from a checkout of the reference
+  sources (``$SQUIDPY_REF``); used only to generate ``tests/golden/*.npz`` (``tests/golden/make_golden*.py``), against
+  which ``tests/test_oracle_vs_reference.py`` and ``tests/test_oracle_golden.py`` pin the restatement.
 
 Pinning status: nhood_enrichment, co_occurrence, Ripley L/F/G and the analytic moments are pinned against the
 running reference code and against golden vectors generated from it (SURVEY.md Appendix A).  Moran's I / Geary's C

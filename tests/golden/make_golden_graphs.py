@@ -1,7 +1,9 @@
 """Generates tests/golden/graphs.npz: outputs of the UNMODIFIED reference graph builders
-(``/root/reference/src/squidpy/gr/neighbors.py``: KNNBuilder, RadiusBuilder, GridBuilder incl. post-processing and the
+(the reference's ``src/squidpy/gr/neighbors.py``: KNNBuilder, RadiusBuilder, GridBuilder incl. post-processing and the
 ``library_key`` block-diagonal combination) on seeded inputs, through the stub-import loader ``oracle/_refload.py``.
-Only runnable in the build container; the output is committed.
+Only runnable where the reference sources are present; the output is committed.  Read it with :func:`load`: float64
+distances are stored as the bitwise XOR with ``sqrt(dx*dx + dy*dy)`` of the coordinates (zero where they agree, which
+compresses to almost nothing), and :func:`load` restores the reference's values bit for bit.
 
     python tests/golden/make_golden_graphs.py
 """
@@ -20,6 +22,7 @@ from oracle import _refload  # noqa: E402
 from tools import synth  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
+PATH = os.path.join(OUT, "graphs.npz")
 
 
 def cases():
@@ -44,6 +47,34 @@ def cases():
     return c
 
 
+def _predicted_bits(co, indptr, indices):
+    """bits of the float64 sqrt(dx*dx + dy*dy) of every stored entry (row of indptr, column in indices)"""
+    r = np.repeat(np.arange(len(indptr) - 1), np.diff(indptr))
+    d = co[r] - co[indices]
+    return np.sqrt(d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]).view(np.uint64)
+
+
+def _coords(gold, prefix):
+    return gold["lib_coords"] if prefix == "lib" else cases()[prefix][0]
+
+
+def _pack(out):
+    """float64 `<prefix>_dst_data` -> `<prefix>_dst_xor`: the bits XOR the predicted distance"""
+    for k in [k for k in out if k.endswith("_dst_data") and out[k].dtype == np.float64]:
+        p = k[: -len("_dst_data")]
+        out[f"{p}_dst_xor"] = out.pop(k).view(np.uint64) ^ _predicted_bits(_coords(out, p), out[f"{p}_dst_indptr"], out[f"{p}_dst_indices"])
+    return out
+
+
+def load() -> dict:
+    """graphs.npz with every `<prefix>_dst_data` as the reference returned it"""
+    gold = dict(np.load(PATH, allow_pickle=False))
+    for k in [k for k in gold if k.endswith("_dst_xor")]:
+        p = k[: -len("_dst_xor")]
+        gold[f"{p}_dst_data"] = (gold.pop(k) ^ _predicted_bits(_coords(gold, p), gold[f"{p}_dst_indptr"], gold[f"{p}_dst_indices"])).view(np.float64)
+    return gold
+
+
 def main():
     import scipy
     import sklearn
@@ -52,7 +83,7 @@ def main():
     # numba cannot type scipy's csr_matrix here (the reference relies on an extension that is not installed): run the
     # reference's own helper un-jitted (same code, interpreted)
     nb._csr_bilateral_diag_scale_helper = nb._csr_bilateral_diag_scale_helper.py_func
-    out = {"meta": np.array(f"numpy {np.__version__}; scipy {scipy.__version__}; sklearn {sklearn.__version__}; reference squidpy @ /root/reference (be17fcf6) gr/neighbors.py")}
+    out = {"meta": np.array(f"numpy {np.__version__}; scipy {scipy.__version__}; sklearn {sklearn.__version__}; reference squidpy (be17fcf6) gr/neighbors.py")}
     for name, (co, cls, kw) in cases().items():
         adj, dst = getattr(nb, cls)(**kw).build(co.copy())
         for tag, m in (("adj", adj), ("dst", dst)):
@@ -75,7 +106,7 @@ def main():
         m = m.tocsr()
         m.sort_indices()
         out[f"lib_{tag}_indptr"], out[f"lib_{tag}_indices"], out[f"lib_{tag}_data"] = m.indptr, m.indices, m.data
-    np.savez_compressed(os.path.join(OUT, "graphs.npz"), **out)
+    np.savez_compressed(PATH, **_pack(out))
     print("wrote graphs.npz", {k: v.shape for k, v in out.items() if k.endswith("adj_data")})
 
 

@@ -1,58 +1,49 @@
-"""Pins the CPU oracle against the UNMODIFIED reference modules (stub import, build container only)."""
+"""Pins the CPU oracle against what the UNMODIFIED reference modules return for the same seeded inputs
+(tests/golden/oracle_reference.npz and the ``grid6_hex`` graph of tests/golden/graphs.npz, both generated from the running
+reference: tests/golden/make_golden_oracle.py, tests/golden/make_golden_graphs.py)."""
 
 from __future__ import annotations
 
+import os
+
 import numpy as np
-import pandas as pd
 import pytest
 
-from oracle import _refload, ref
+from oracle import ref
+from tests.golden.make_golden_oracle import NHOOD_CASES, NHOOD_PERMS, NHOOD_SEED, cooc_case, interaction_cases, nhood_case
 from tools import synth
 
-pytestmark = pytest.mark.skipif(not _refload.available(), reason="/root/reference not present (GPU box)")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
-def refmods():
-    return _refload.load(morans_i=ref.morans_i, gearys_c=ref.gearys_c)
+def gold():
+    return dict(np.load(os.path.join(GOLDEN, "oracle_reference.npz"), allow_pickle=False))
 
 
-def test_hex_graph_matches_gridbuilder(refmods):
-    co = synth.hex_coords(23, 31)
-    adj, _ = refmods["nb"].GridBuilder(n_neighs=6).build(co)
+def test_hex_graph_matches_gridbuilder():
+    gold = np.load(os.path.join(GOLDEN, "graphs.npz"), allow_pickle=False)  # GridBuilder(n_neighs=6) on hex_coords(23, 31)
     g = synth.hex_graph(23, 31)
-    assert adj.nnz == g.nnz and (adj != g).nnz == 0
+    np.testing.assert_array_equal(g.indptr, gold["grid6_hex_adj_indptr"])
+    np.testing.assert_array_equal(g.indices, gold["grid6_hex_adj_indices"])
+    np.testing.assert_array_equal(g.data, gold["grid6_hex_adj_data"])
     assert g.dtype == np.float32 and g.indices.dtype == np.int32
 
 
-@pytest.mark.parametrize("n_cls,libs", [(2, False), (7, False), (30, True)])
-def test_nhood_perms_vs_reference(refmods, n_cls, libs):
-    nh = refmods["nh"]
-    g = synth.hex_graph(37, 41)
-    n = g.shape[0]
-    lab = np.random.default_rng(n_cls).integers(0, n_cls, n).astype(np.uint32)
-    ind, ptr = g.indices.astype(np.uint32), g.indptr.astype(np.uint32)
-    fn = nh._create_function(n_cls)
-    np.testing.assert_array_equal(ref.nhood_count(ptr, ind, lab, n_cls), fn(ind, ptr, lab))
-    libraries = pd.Series(pd.Categorical(np.random.default_rng(1).integers(0, 3, n).astype(str))) if libs else None
-    gens = refmods["utils"].spawn_generators(11, 12)
-    exp = nh._nhood_enrichment_helper(list(range(12)), fn, ind, ptr, lab, libraries, n_cls, gens)
-    got = ref.nhood_perm_counts(ptr, ind, lab, n_cls, ref.spawn_states(11, 12),
+@pytest.mark.parametrize("n_cls,libs", NHOOD_CASES)
+def test_nhood_perms_vs_reference(gold, n_cls, libs):
+    ptr, ind, lab, libraries = nhood_case(n_cls, libs)
+    np.testing.assert_array_equal(ref.nhood_count(ptr, ind, lab, n_cls), gold[f"nhood{n_cls}_count"])
+    got = ref.nhood_perm_counts(ptr, ind, lab, n_cls, ref.spawn_states(NHOOD_SEED, NHOOD_PERMS),
                                 None if libraries is None else libraries.cat.codes.to_numpy(), 3 if libs else 0)
-    np.testing.assert_array_equal(got, exp.astype(np.uint32))
+    np.testing.assert_array_equal(got, gold[f"nhood{n_cls}_perms"])
 
 
-def test_cooc_vs_reference(refmods):
-    pp = refmods["pp"]
-    rr = np.random.default_rng(5)
-    pts = (rr.random((1500, 2)) * 300).astype(np.float32)
-    lb = rr.integers(0, 5, 1500).astype(np.int32)
-    iv = np.linspace(1, 200, 20, dtype=np.float32)
-    exp = pp._occur_count(pts[:, 0].copy(), pts[:, 1].copy(), iv[1:] ** 2, lb, 1500, 5, 19)
-    np.testing.assert_array_equal(ref.occur_count(pts[:, 0], pts[:, 1], iv[1:] ** 2, lb, 5), exp)
-    occ_ref = pp._co_occurrence_helper(pts[:, 0].copy(), pts[:, 1].copy(), iv, lb)
+def test_cooc_vs_reference(gold):
+    pts, lb, iv = cooc_case()
+    np.testing.assert_array_equal(ref.occur_count(pts[:, 0], pts[:, 1], iv[1:] ** 2, lb, 5), gold["cooc_counts"])
     occ, _ = ref.co_occurrence_helper(pts[:, 0], pts[:, 1], iv, lb)
-    np.testing.assert_allclose(occ, occ_ref, rtol=1e-12)
+    np.testing.assert_allclose(occ, gold["cooc_occ"], rtol=1e-12)
 
 
 def test_pair_counts_vs_sklearn():
@@ -64,7 +55,7 @@ def test_pair_counts_vs_sklearn():
     np.testing.assert_array_equal(ref.pair_counts(P, sup), KDTree(P).two_point_correlation(P, sup, dualtree=True))
 
 
-def test_interaction_matrix_oracle_kat_and_reference():
+def test_interaction_matrix_oracle_kat_and_reference(gold):
     """Oracle restatement of interaction_matrix (next row of SURVEY 8f): the reference's own known answers
     (tests/graph/test_nhood.py:153-173, fixture tests/conftest.py:177-194) and its numba kernel on random graphs."""
     import scipy.sparse as sp
@@ -79,17 +70,8 @@ def test_interaction_matrix_oracle_kat_and_reference():
     assert ref.interaction_matrix(g, codes, 2).dtype == np.int64
     np.testing.assert_allclose(ref.interaction_matrix(g, codes, 2, normalized=True).sum(1), 1.0)
 
-    if not _refload.available():
-        pytest.skip("reference sources not present (GPU box)")
-    kern = _refload.load()["nh"]._interaction_matrix
-    rng = np.random.default_rng(0)
-    for n, dens, k in ((200, 0.05, 5), (1500, 0.004, 12)):
-        a = sp.random(n, n, density=dens, format="csr", random_state=int(rng.integers(1 << 30)), dtype=np.float32)
-        codes = rng.integers(0, k, n)
+    for name, a, codes, k in interaction_cases():
         for weights in (False, True):
-            data = a.data if weights else np.broadcast_to(1, shape=len(a.data))
-            exp = np.zeros((k, k), dtype=float)
-            kern(np.ascontiguousarray(data), a.indices, a.indptr, codes, exp)
             got = ref.interaction_matrix(a, codes, k, weights=weights)
             assert got.dtype == np.float64
-            np.testing.assert_array_equal(got, exp)  # same accumulation order: bit-identical float sums
+            np.testing.assert_array_equal(got, gold[f"interaction_{name}_w{int(weights)}"])  # same accumulation order: bit-identical float sums
