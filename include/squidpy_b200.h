@@ -137,15 +137,11 @@ int sqb_nhood_shuffled_labels(sqb_nhood* h, int64_t p0, int64_t p1, uint32_t* ou
 
 /* Tuning / test options (all variants produce bit-identical results).
  *   "shuffle_algo"   -1 auto [default]: two-kernel list replay (7) for many permutations of large arrays, else 1 / 2;
- *                    1 CTA per permutation; 2 warp per permutation; 7 two kernels (swap-target generation + list apply).
- *                    0 (serial), 3 (large windows), 4 (two-warp pipeline), 5 (two kernels, ordered replay), 6 (fused list
- *                    kernel) and 8 (region replay: every random access in shared memory, one region of the array per pass)
- *                    are superseded / slower cross-check variants compiled into the TEST build only (make testvariants);
- *                    the product library answers SQB_ERR_UNSUPPORTED for them.
+ *                    1 CTA per permutation; 2 warp per permutation; 7 two kernels (swap-target generation + list apply);
+ *                    any other value is rejected with SQB_ERR_INVALID.
  *   "shuffle_threads" 128/256/512/1024 (algos 1, 7), "shuffle_r" 2/4/8 steps per thread (7),
  *   "shuffle_q"      1/2/4/8 PCG64 outputs per lane and batch (2, and the target generation of 7),
  *   "shuffle_low"    elements of every label array kept in shared memory by the apply kernel of 7 (-1 all that fits, 0 off),
- *   "shuffle_region" positions per region of 8 (0 = as many as shared memory holds; smaller values are a test hook),
  *   "shuffle_ctas"   persistent grid size = permutations in flight (0 = occupancy x SM count),
  *   "shuffle_stagger_us" start-up stagger of the persistent CTAs, "shuffle_wfactor_x100" window = min(i/4, f*sqrt(i)),
  *   "perm_chunk"     permutations resident at once (read at the next upload), "count_algo" 0 auto / 1 shared-memory histograms /

@@ -13,9 +13,7 @@ import threading
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# $SQB_LIB_PATH: another build of the same C ABI (the test suite points it at the build that also contains the superseded
-# replay variants, tests/native/libsquidpy_b200_testvariants.so); the package itself only ever ships libsquidpy_b200.so
-LIB_PATH = os.environ.get("SQB_LIB_PATH") or os.path.join(_HERE, "libsquidpy_b200.so")
+LIB_PATH = os.path.join(_HERE, "libsquidpy_b200.so")
 ABI_VERSION = 3
 
 _lock = threading.Lock()

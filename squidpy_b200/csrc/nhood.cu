@@ -11,8 +11,9 @@
 //                          Fisher-Yates target of every step to J[P][stride]
 //      nhood_apply_list    one CTA per permutation applies the swaps in 2048-step windows: 2-bit duplicate filter,
 //                          per-position lists instead of an ordered replay of conflicting swaps, low part of the array in
-//                          shared memory, next window marked while the current one is resolved (sections 2f-2h; 2a-2e
-//                          are the earlier, bit-identical variants kept as options and cross-checks)
+//                          shared memory, next window marked while the current one is resolved (sections 2c-2e)
+//      nhood_shuffle_cta   replace the two kernels above for few permutations (one CTA each, 2a) or many permutations of
+//      nhood_shuffle_warp  small arrays (one warp each, 2b): one kernel replays the stream and applies the swaps
 //   3. nhood_transpose     [P][n] -> [PB/32][n + 1][32] (groups of 32 permutations, permutation-minor inside a group) so that
 //                          one warp lane = one permutation and a CTA's labels of consecutive nodes are contiguous
 //   4. nhood_count         CSR neighbour-pair histogram: lane = permutation, warp walks the CSR once for 32
@@ -32,7 +33,6 @@ typedef unsigned __int128 u128;
 // (and ptxas turns a `bar.warp.sync 0xffffffff` it considers redundant into a NOP, so the full mask is passed in
 // at run time, as a kernel argument, which it cannot reason about).
 #define SQB_CONVERGE() asm volatile("bar.warp.sync %0;" ::"r"(full_mask) : "memory")
-#define SQB_CONVERGE_W() __syncwarp()
 
 __constant__ uint64_t c_jump_M[SQB_PCG_JUMP_BITS][2] = SQB_PCG_JUMP_M_INIT;
 __constant__ uint64_t c_jump_C[SQB_PCG_JUMP_BITS][2] = SQB_PCG_JUMP_C_INIT;
@@ -63,50 +63,6 @@ __device__ __forceinline__ void pcg_jump_consts(uint64_t d, u128& M, u128& C) {
     }
 }
 
-#define PCG_MULT_HI 0x2360ED051FC65DA4ULL
-#define PCG_MULT_LO 0x4385DF649FCCF645ULL
-
-struct PcgSerial {
-    u128 state, inc;
-    int has32;
-    uint32_t buf;
-    __device__ __forceinline__ uint64_t next64() {
-        state = state * mk128(PCG_MULT_HI, PCG_MULT_LO) + inc;
-        return pcg_output(state);
-    }
-    __device__ __forceinline__ uint32_t next32() {
-        if (has32) {
-            has32 = 0;
-            return buf;
-        }
-        uint64_t v = next64();
-        has32 = 1;
-        buf = (uint32_t)(v >> 32);
-        return (uint32_t)v;
-    }
-    __device__ __forceinline__ uint64_t interval(uint64_t max) {
-        if (max == 0) return 0;
-        uint64_t mask = max;
-        mask |= mask >> 1;
-        mask |= mask >> 2;
-        mask |= mask >> 4;
-        mask |= mask >> 8;
-        mask |= mask >> 16;
-        mask |= mask >> 32;
-        uint64_t v;
-        if (max <= 0xffffffffULL) {
-            do {
-                v = next32() & mask;
-            } while (v > max);
-        } else {
-            do {
-                v = next64() & mask;
-            } while (v > max);
-        }
-        return v;
-    }
-};
-
 // ------------------------------------------------------------------------------------------------
 // 1. fill: labels[p][0..stride) = base[0..stride)   (16-byte vectors; stride*sizeof(LT) % 16 == 0)
 // ------------------------------------------------------------------------------------------------
@@ -120,36 +76,8 @@ __global__ void nhood_fill_kernel(uint4* __restrict__ dst, const uint4* __restri
     }
 }
 
-#ifdef SQB_TEST_VARIANTS  // superseded replay variant: compiled into the test build only (tests/native/libsquidpy_b200_testvariants.so)
 // ------------------------------------------------------------------------------------------------
-// 2a. reference-style serial replay: one thread per permutation (cross-check / fallback option)
-// ------------------------------------------------------------------------------------------------
-template <typename LT>
-__global__ void nhood_shuffle_serial_kernel(LT* __restrict__ labels, int64_t stride, const uint64_t* __restrict__ states,
-                                            int64_t n_perms, int nseg, const int64_t* __restrict__ seg_start,
-                                            const int64_t* __restrict__ seg_len) {
-    int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (p >= n_perms) return;
-    PcgSerial g;
-    g.state = mk128(states[p * 4 + 0], states[p * 4 + 1]);
-    g.inc = mk128(states[p * 4 + 2], states[p * 4 + 3]);
-    g.has32 = 0;
-    g.buf = 0;
-    LT* a = labels + p * stride;
-    for (int s = 0; s < nseg; ++s) {
-        LT* b = a + seg_start[s];
-        for (int64_t i = seg_len[s] - 1; i >= 1; --i) {
-            int64_t j = (int64_t)g.interval((uint64_t)i);
-            LT t = b[i];
-            b[i] = b[j];
-            b[j] = t;
-        }
-    }
-}
-
-#endif  // SQB_TEST_VARIANTS
-// ------------------------------------------------------------------------------------------------
-// 2b. CTA-parallel exact replay of numpy Generator.shuffle (see file header; validated step by step against
+// 2a. CTA-parallel exact replay of numpy Generator.shuffle (see file header; validated step by step against
 //     numpy by the Python emulation tests/emu_shuffle.py).
 //
 //  Raw stream: v_{2k} = lo32(out_k), v_{2k+1} = hi32(out_k)  (pcg64_next32 hands out the low half first).
@@ -441,11 +369,12 @@ __global__ void __launch_bounds__(NT) nhood_shuffle_cta_kernel(LT* __restrict__ 
 }
 
 // ------------------------------------------------------------------------------------------------
-// 2c. WARP-per-permutation exact replay (default).  Same algorithm as 2b, but every synchronisation is warp level
-//     (ballots, shuffles, __syncwarp): no block barriers at all.  A lane owns Q consecutive-by-32 PCG64 outputs
-//     (2Q raw 32-bit values) per batch and executes the Fisher-Yates steps of the values IT drew; the swaps act on
-//     global memory directly (L2): conflict-free steps in parallel, conflicting ones (own-range targets, duplicate
-//     targets found through a per-warp shared-memory hash table) afterwards by lane 0 in step order.
+// 2b. WARP-per-permutation exact replay (the auto choice for many permutations of arrays under 65 536 elements).
+//     Same algorithm as 2a, but every synchronisation is warp level (ballots, shuffles, __syncwarp): no block barriers
+//     at all.  A lane owns Q consecutive-by-32 PCG64 outputs (2Q raw 32-bit values) per batch and executes the
+//     Fisher-Yates steps of the values IT drew; the swaps act on global memory directly (L2): conflict-free steps in
+//     parallel, conflicting ones (own-range targets, duplicate targets found through a per-warp shared-memory hash
+//     table) afterwards by lane 0 in step order.
 //     ~4 warp instructions per shuffle step instead of ~12 for the CTA version, and thousands of permutations in
 //     flight per GPU, so the random label accesses of different permutations overlap.
 // ------------------------------------------------------------------------------------------------
@@ -648,309 +577,19 @@ __global__ void __launch_bounds__(128) nhood_shuffle_warp_kernel(LT* __restrict_
     }
 }
 
-#ifdef SQB_TEST_VARIANTS  // superseded replay variant: compiled into the test build only (tests/native/libsquidpy_b200_testvariants.so)
 // ------------------------------------------------------------------------------------------------
-// 2d. CTA per permutation, LARGE windows (default for big n).  ncu showed 2b/2c to be bound by the dependent
-//     instruction chain of a window (~600-1200 instructions per warp per window at IPC ~0.1-0.3), not by HBM or issue
-//     slots, so this version (a) makes a window R x larger (every thread draws R PCG64 outputs = 2R raw values per
-//     batch and executes the Fisher-Yates steps of the values IT drew, the per-value work being independent chains),
-//     (b) swaps conflict-free steps straight in global memory and stages only the conflicting ones in shared memory
-//     for the ordered replay, (c) needs 8-9 block barriers per ~3000 steps instead of per ~750.
-// ------------------------------------------------------------------------------------------------
-template <typename LT, int NT, int R>
-__global__ void __launch_bounds__(NT) nhood_shuffle_cta2_kernel(LT* __restrict__ labels, int64_t stride,
-                                                                const uint64_t* __restrict__ states, int64_t n_perms,
-                                                                int nseg, const int64_t* __restrict__ seg_start,
-                                                                const int64_t* __restrict__ seg_len, float wfactor,
-                                                                uint32_t full_mask, uint64_t stagger_ns) {
-    constexpr int V = 2 * R;          // raw values per thread per batch
-    constexpr int RAW = V * NT;       // raw values per batch
-    constexpr int HS = 2 * RAW;       // hash slots (load factor <= 0.5), power of two
-    constexpr int NW = NT / 32;
-    constexpr int LOG_HS = (HS == 1024 ? 10 : HS == 2048 ? 11 : HS == 4096 ? 12 : HS == 8192 ? 13 : HS == 16384 ? 14 : 15);
-    static_assert(HS == (1 << LOG_HS), "HS must be a power of two");
-    constexpr int HS_SHIFT = 32 - LOG_HS;
-
-    extern __shared__ __align__(16) unsigned char sqb_shuffle_smem[];
-    unsigned long long* s_tab = reinterpret_cast<unsigned long long*>(sqb_shuffle_smem);  // (target << 32) | step, or EMPTY
-    uint32_t* s_sj = reinterpret_cast<uint32_t*>(s_tab + HS);
-    uint32_t* s_flag = s_sj + RAW;
-    int* s_wsum = reinterpret_cast<int*>(s_flag + RAW / 32);  // [R][32]
-    int* s_misc = s_wsum + R * 32;                             // [4]
-    LT* s_own = reinterpret_cast<LT*>(s_misc + 4);
-    LT* s_hval = s_own + RAW;
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-    for (int h = tid; h < HS; h += NT) s_tab[h] = SQB_EMPTY64;
-    for (int w = tid; w < RAW / 32; w += NT) s_flag[w] = 0;
-    for (int w = tid; w < R * 32; w += NT) s_wsum[w] = 0;
-    if (tid < 4) s_misc[tid] = 0;
-    u128 Mn, Cn, Mt, Ct;
-    pcg_jump_consts((uint64_t)NT, Mn, Cn);
-    pcg_jump_consts((uint64_t)tid + 1, Mt, Ct);
-    sqb_stagger(stagger_ns * blockIdx.x / gridDim.x);
-    __syncthreads();
-
-    for (int64_t perm = blockIdx.x; perm < n_perms; perm += gridDim.x) {
-        LT* __restrict__ a = labels + perm * stride;
-        const uint64_t* st4 = states + perm * 4;
-        const u128 inc = mk128(st4[2], st4[3]);
-        u128 st = Mt * mk128(st4[0], st4[1]) + Ct * inc;  // state of output index `tid`
-        const u128 Cn_inc = Cn * inc;
-        uint32_t raw[V];
-#pragma unroll
-        for (int k = 0; k < V; ++k) raw[k] = 0;
-        int pos = RAW;
-
-        for (int seg = 0; seg < nseg; ++seg) {
-            const int64_t base = seg_start[seg];
-            int i_cur = (int)(seg_len[seg] - 1);  // n < 2^31
-            while (i_cur >= 1) {
-                if (pos >= RAW) {
-#pragma unroll
-                    for (int q = 0; q < R; ++q) {  // output q*NT + tid of this batch -> raw 2*(q*NT+tid) + {0,1}
-                        const uint64_t o = pcg_output(st);
-                        st = Mn * st + Cn_inc;
-                        raw[2 * q] = (uint32_t)o;
-                        raw[2 * q + 1] = (uint32_t)(o >> 32);
-                    }
-                    pos = 0;
-                }
-                const uint32_t mask = 0xFFFFFFFFu >> __clz(i_cur);
-                const int i_lo = (int)(mask >> 1) + 1;
-                const int n_ph = i_cur - i_lo + 1;
-                const int K = sqb_window_size((int64_t)i_cur, RAW - pos, RAW, wfactor);
-                uint32_t inmask = 0, fmask = 0;  // bit k: value k inside the window / accepted
-#pragma unroll
-                for (int k = 0; k < V; ++k) {
-                    const int r = (k >> 1) * (2 * NT) + 2 * tid + (k & 1);
-                    if (r >= pos && r < pos + K) {
-                        inmask |= 1u << k;
-                        if ((raw[k] & mask) <= (uint32_t)i_cur) fmask |= 1u << k;
-                    }
-                }
-                // ---- acceptance fixed point; c(k) = cb[k>>1] + (k odd ? bit(k-1) : 0) ----
-                int cb[R];
-                int total = 0;
-                while (true) {
-                    uint32_t blo[R], bhi[R];
-#pragma unroll
-                    for (int q = 0; q < R; ++q) {
-                        blo[q] = __ballot_sync(0xffffffffu, (fmask >> (2 * q)) & 1u);
-                        bhi[q] = __ballot_sync(0xffffffffu, (fmask >> (2 * q + 1)) & 1u);
-                        if (lane == 0) s_wsum[q * 32 + warp] = __popc(blo[q]) + __popc(bhi[q]);
-                    }
-                    __syncthreads();
-                    int run = 0;
-#pragma unroll
-                    for (int q = 0; q < R; ++q) {
-                        const int v = (lane < NW) ? s_wsum[q * 32 + lane] : 0;
-                        int incl = v;
-#pragma unroll
-                        for (int d = 1; d < 32; d <<= 1) {
-                            const int t = __shfl_up_sync(0xffffffffu, incl, d);
-                            if (lane >= d) incl += t;
-                        }
-                        const int woff = __shfl_sync(0xffffffffu, incl - v, warp);
-                        const int tot = __shfl_sync(0xffffffffu, incl, 31);
-                        cb[q] = run + woff + __popc(blo[q] & lt_mask) + __popc(bhi[q] & lt_mask);
-                        run += tot;
-                    }
-                    total = run;
-                    uint32_t nf = 0;
-#pragma unroll
-                    for (int k = 0; k < V; ++k) {
-                        const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                        const uint32_t uk = raw[k] & mask;
-                        if (((inmask >> k) & 1u) && uk <= (uint32_t)i_cur && (int)uk <= i_cur - ck) nf |= 1u << k;
-                    }
-                    const int any = __syncthreads_or(nf != fmask);
-                    if (!any) break;
-                    fmask = nf;
-                }
-                const bool phase_ends = total >= n_ph;
-                const int S = phase_ends ? n_ph : total;
-                const int own_lo = i_cur - S;
-                // ---- B1: conflict detection (steps are executed by the thread that drew them) ----
-                uint32_t actmask = 0, insmask = 0;
-                bool any_flag_local = false;
-                uint32_t slotv[V];  // hash slot of every key this thread inserted
-#pragma unroll
-                for (int k = 0; k < V; ++k) slotv[k] = 0;
-#pragma unroll
-                for (int k = 0; k < V; ++k) {
-                    if ((fmask >> k) & 1u) {
-                        const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                        if (phase_ends && ck == S - 1) s_misc[0] = (k >> 1) * (2 * NT) + 2 * tid + (k & 1);
-                        if (ck < S) {
-                            const uint32_t j = raw[k] & mask;
-                            s_sj[ck] = j;
-                            if ((int)j > own_lo) {
-                                const int s2 = i_cur - (int)j;
-                                if (s2 != ck) {
-                                    actmask |= 1u << k;
-                                    atomicOr(&s_flag[ck >> 5], 1u << (ck & 31));
-                                    atomicOr(&s_flag[s2 >> 5], 1u << (s2 & 31));
-                                }
-                            } else {
-                                actmask |= 1u << k;
-                                uint32_t h = (j * 2654435761u) >> HS_SHIFT;
-                                const unsigned long long mine = ((unsigned long long)j << 32) | (unsigned)ck;
-                                while (true) {
-                                    const unsigned long long prev = atomicCAS(&s_tab[h], SQB_EMPTY64, mine);
-                                    if (prev == SQB_EMPTY64) {
-                                        insmask |= 1u << k;
-                                        slotv[k] = h;
-                                        break;
-                                    }
-                                    if ((uint32_t)(prev >> 32) == j) {
-                                        const int so = (int)(uint32_t)prev;
-                                        atomicOr(&s_flag[ck >> 5], 1u << (ck & 31));
-                                        atomicOr(&s_flag[so >> 5], 1u << (so & 31));
-                                        break;
-                                    }
-                                    h = (h + 1) & (HS - 1);
-                                }
-                            }
-                        }
-                    }
-                }
-                SQB_CONVERGE();
-                __syncthreads();
-                const int newpos = phase_ends ? (s_misc[0] + 1) : (pos + K);
-                // ---- B2: conflict-free steps swap directly in global memory; conflicting ones are staged ----
-                // Written branch-free (ternaries / single-statement ifs => predicated loads and stores): compute-sanitizer
-                // synccheck showed lanes arriving at the next block barrier un-converged when this phase contained
-                // real branches around the global loads (cudaErrorIllegalInstruction on sm_100).
-                uint32_t direct = 0, staged = 0;
-                {
-                    LT vi[V], vj[V];
-#pragma unroll
-                    for (int k = 0; k < V; ++k) {
-                        const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                        const bool live = ((fmask >> k) & 1u) && ck < S;
-                        const int cks = live ? ck : 0;
-                        const bool flagged = live && ((s_flag[cks >> 5] >> (cks & 31)) & 1u);
-                        const bool dir = live && !flagged && ((actmask >> k) & 1u);
-                        const bool ins = (insmask >> k) & 1u;
-                        staged |= (flagged ? 1u : 0u) << k;  // includes self swaps that another step targets
-                        direct |= (dir ? 1u : 0u) << k;
-                        const uint32_t j = raw[k] & mask;
-                        const LT* po = a + base + (i_cur - cks);
-                        const LT* pt = a + base + (int64_t)((dir || (flagged && ins)) ? j : 0u);
-                        vi[k] = (dir || flagged) ? ld_cs<LT>(po) : (LT)0;
-                        vj[k] = (dir || (flagged && ins)) ? ld_cg<LT>(pt) : (LT)0;
-                    }
-                    any_flag_local = staged != 0;
-#pragma unroll
-                    for (int k = 0; k < V; ++k) {
-                        const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                        const bool dir = (direct >> k) & 1u, stg = (staged >> k) & 1u, ins = (insmask >> k) & 1u;
-                        const int cks = (dir || stg) ? ck : 0;
-                        const uint32_t j = raw[k] & mask;
-                        if (dir) st_cs<LT>(a + base + (i_cur - cks), vj[k]);  // final position: never read again here
-                        if (dir) a[base + (int64_t)j] = vi[k];
-                        if (stg) s_own[cks] = vi[k];
-                        if (stg && ins) s_hval[slotv[k]] = vj[k];
-                    }
-                }
-                // block-wide OR through shared memory + a plain barrier: bar.red (__syncthreads_or) is a warp-aligned
-                // instruction and faults ("divergent thread(s) in warp") when the lanes that took the staging / probing
-                // paths above have not re-converged, which ptxas does not guarantee here
-                if (any_flag_local) s_misc[1] = 1;
-                SQB_CONVERGE();
-                __syncthreads();
-                const int any_flag = s_misc[1];
-                if (any_flag) {
-                    // ---- B3: ordered replay of the conflicting steps on the staged values (warp 0, lane 0) ----
-                    if (warp == 0) {
-                        const int nwords = (S + 31) >> 5;
-                        for (int wb = 0; wb < nwords; wb += 32) {
-                            const uint32_t myw = (wb + lane < nwords) ? s_flag[wb + lane] : 0u;
-                            uint32_t nz = __ballot_sync(0xffffffffu, myw != 0u);
-                            while (nz) {
-                                const int wl = __ffs(nz) - 1;
-                                nz &= nz - 1;
-                                uint32_t bits = __shfl_sync(0xffffffffu, myw, wl);
-                                if (lane == 0) {
-                                    while (bits) {
-                                        const int b = __ffs(bits) - 1;
-                                        bits &= bits - 1;
-                                        const int s = (wb + wl) * 32 + b;
-                                        const uint32_t j = s_sj[s];
-                                        const LT x = s_own[s];
-                                        if ((int)j > own_lo) {
-                                            const int s2 = i_cur - (int)j;
-                                            if (s2 != s) {
-                                                const LT y = s_own[s2];
-                                                s_own[s] = y;
-                                                s_own[s2] = x;
-                                            }
-                                        } else {
-                                            uint32_t h = (j * 2654435761u) >> HS_SHIFT;
-                                            while ((uint32_t)(s_tab[h] >> 32) != j) h = (h + 1) & (HS - 1);
-                                            const LT y = s_hval[h];
-                                            s_own[s] = y;
-                                            s_hval[h] = x;
-                                        }
-                                    }
-                                }
-                            }
-                        }
-                    }
-                    __syncthreads();
-                    // ---- B4: write the staged values back ----
-#pragma unroll
-                    for (int k = 0; k < V; ++k) {
-                        const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                        const bool stg = (staged >> k) & 1u, ins = (insmask >> k) & 1u;
-                        const int cks = stg ? ck : 0;
-                        const uint32_t j = raw[k] & mask;
-                        if (stg) st_cs<LT>(a + base + (i_cur - cks), s_own[cks]);
-                        if (stg && ins) a[base + (int64_t)j] = s_hval[slotv[k]];
-                    }
-                    SQB_CONVERGE();
-                    __syncthreads();
-                    for (int w = tid; w < ((S + 31) >> 5); w += NT) s_flag[w] = 0;
-                }
-                // reset the hash table entries this thread inserted
-#pragma unroll
-                for (int k = 0; k < V; ++k)
-                    if ((insmask >> k) & 1u) s_tab[slotv[k]] = SQB_EMPTY64;
-                SQB_CONVERGE();
-                __syncthreads();
-                if (tid == 0) s_misc[1] = 0;  // next writers come after the next window's barriers
-                i_cur -= S;
-                pos = newpos;
-            }
-        }
-    }
-}
-
-#endif  // SQB_TEST_VARIANTS
-// ------------------------------------------------------------------------------------------------
-// 2g. CTA-per-permutation replay WITHOUT a serial pass ("list" kernel, shuffle_algo 6).
-//     Measured on B200 (tools/micro/rmw_bench.cu): random byte swaps over label arrays that stay inside the 126 MB L2
-//     run at ~55 G swaps/s (18 ms per 1e9 steps), over 1000 arrays (1 GB) at ~20 G swaps/s, because every swap then
-//     costs two random 32-byte DRAM sectors.  So the fast regime is FEW permutations in flight (<= ~150-250 label
-//     arrays, one per CTA) and each of them replayed as fast as possible; 2b/2d in that regime were bound by window
-//     latency: ~10 block barriers, an exposed global round trip and a one-thread ordered replay of the conflicting
-//     steps per window.  This kernel removes those:
-//       * the window's global loads (own range, cooperatively; random targets for every optimistically accepted
-//         value) are issued BEFORE the acceptance fixed point, whose barriers hide their latency;
-//       * acceptance iterations cost one barrier each (double-buffered warp sums, monotonic change stamp);
-//       * conflicts are not serialised.  Every step pushes itself on the list of the position it targets (outside
-//         targets: shared-memory hash table keyed by position; targets inside the window's own range: one list head per
-//         step).  With T(s) = value of step s's top position just before step s
-//                          = T(latest earlier step targeting that top) or its ORIGINAL value,
-//         step s writes a[top_s] = value of position j_s just before step s
-//                                = T(latest earlier step targeting j_s) or the original a[j_s],
-//         and the last step targeting an outside position p writes a[p] = T(that step).  Only original values are
-//         read, all lists are immutable once built, so every step resolves independently (chains are almost always
-//         empty) and windows can be several times larger than with an ordered replay
-//         (tests/emu_shuffle.py::resolve_window_lists is the executable specification).
-//     Barriers per window: (acceptance iterations + 1) + 2.
+// 2c. List-based resolution of the conflicts inside a window of Fisher-Yates steps (used by the apply kernel, 2e).
+//     Swaps of one window commute unless they share a position.  Instead of replaying the conflicting ones in step
+//     order, every step pushes itself on the list of the position it targets (outside targets: shared-memory hash table
+//     keyed by position; targets inside the window's own range: one list head per step).  With
+//       T(s) = value of step s's top position just before step s
+//            = T(latest earlier step targeting that top) or its ORIGINAL value,
+//     step s writes a[top_s] = value of position j_s just before step s
+//                            = T(latest earlier step targeting j_s) or the original a[j_s],
+//     and the last step targeting an outside position p writes a[p] = T(that step).  Only original values are read, all
+//     lists are immutable once built, so every step resolves independently (chains are almost always empty) and windows
+//     can be several times larger than with an ordered replay (tests/emu_shuffle.py::resolve_window_lists is the
+//     executable specification).
 // ------------------------------------------------------------------------------------------------
 #define SQB_NONE16 0xFFFFu
 #define SQB_NONE32 0xFFFFFFFFu
@@ -986,539 +625,15 @@ __device__ __forceinline__ int sqb_list_latest_before(const uint16_t* __restrict
     return best;
 }
 
-#ifdef SQB_TEST_VARIANTS  // superseded replay variant: compiled into the test build only (tests/native/libsquidpy_b200_testvariants.so)
-template <typename LT, int NT, int R>
-__global__ void __launch_bounds__(NT) nhood_shuffle_list_kernel(LT* __restrict__ labels, int64_t stride,
-                                                                const uint64_t* __restrict__ states, int64_t n_perms,
-                                                                int nseg, const int64_t* __restrict__ seg_start,
-                                                                const int64_t* __restrict__ seg_len, float wfactor,
-                                                                uint32_t full_mask, uint64_t stagger_ns) {
-    constexpr int V = 2 * R;     // raw values per thread per batch
-    constexpr int RAW = V * NT;  // raw values per batch = max steps per window
-    constexpr int HS = 2 * RAW;  // hash slots (load factor <= 0.5), power of two
-    constexpr int NW = NT / 32;
-    constexpr int LOG_HS = (HS == 1024 ? 10 : HS == 2048 ? 11 : HS == 4096 ? 12 : HS == 8192 ? 13 : HS == 16384 ? 14 : 15);
-    static_assert(HS == (1 << LOG_HS), "HS must be a power of two");
-    static_assert(RAW < 0xFFFF, "step indices are stored in 16 bits");
-    constexpr int HS_SHIFT = 32 - LOG_HS;
-
-    extern __shared__ __align__(16) unsigned char sqb_shuffle_smem[];
-    unsigned long long* s_tab = reinterpret_cast<unsigned long long*>(sqb_shuffle_smem);  // (target << 32) | list head, or EMPTY
-    uint32_t* s_ohead = reinterpret_cast<uint32_t*>(s_tab + HS);                            // [RAW] head of "steps targeting top of u"
-    int* s_wsum = reinterpret_cast<int*>(s_ohead + RAW);                                    // [2][R][32]
-    int* s_misc = s_wsum + 2 * R * 32;                                                      // [0] r*, [1] change stamp
-    uint16_t* s_next = reinterpret_cast<uint16_t*>(s_misc + 4);                             // [RAW] list links
-    LT* s_otop = reinterpret_cast<LT*>(s_next + RAW);                                       // [RAW] original own-range values
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-    for (int h = tid; h < HS; h += NT) s_tab[h] = SQB_EMPTY64;
-    for (int w = tid; w < RAW; w += NT) s_ohead[w] = SQB_NONE32;
-    for (int w = tid; w < 2 * R * 32; w += NT) s_wsum[w] = 0;
-    if (tid < 4) s_misc[tid] = 0;
-    u128 Mn, Cn, Mt, Ct;
-    pcg_jump_consts((uint64_t)NT, Mn, Cn);
-    pcg_jump_consts((uint64_t)tid + 1, Mt, Ct);
-    int stamp = 0;  // acceptance iteration counter (uniform across the CTA, monotonic for the whole kernel)
-    sqb_stagger(stagger_ns * blockIdx.x / gridDim.x);
-    __syncthreads();
-
-    for (int64_t perm = blockIdx.x; perm < n_perms; perm += gridDim.x) {
-        LT* __restrict__ a = labels + perm * stride;
-        const uint64_t* st4 = states + perm * 4;
-        const u128 inc = mk128(st4[2], st4[3]);
-        u128 st = Mt * mk128(st4[0], st4[1]) + Ct * inc;  // state of output index `tid`
-        const u128 Cn_inc = Cn * inc;
-        uint32_t raw[V];
-#pragma unroll
-        for (int k = 0; k < V; ++k) raw[k] = 0;
-        int pos = RAW;
-
-        for (int seg = 0; seg < nseg; ++seg) {
-            const int64_t base = seg_start[seg];
-            int i_cur = (int)(seg_len[seg] - 1);  // n < 2^31
-            while (i_cur >= 1) {
-                if (pos >= RAW) {
-#pragma unroll
-                    for (int q = 0; q < R; ++q) {  // output q*NT + tid of this batch -> raw 2*(q*NT+tid) + {0,1}
-                        const uint64_t o = pcg_output(st);
-                        st = Mn * st + Cn_inc;
-                        raw[2 * q] = (uint32_t)o;
-                        raw[2 * q + 1] = (uint32_t)(o >> 32);
-                    }
-                    pos = 0;
-                }
-                const uint32_t mask = 0xFFFFFFFFu >> __clz(i_cur);
-                const int i_lo = (int)(mask >> 1) + 1;
-                const int n_ph = i_cur - i_lo + 1;
-                const int K = sqb_window_size((int64_t)i_cur, RAW - pos, RAW, wfactor);
-                uint32_t inmask = 0, fmask = 0;  // bit k: value k inside the window / accepted (optimistic start)
-#pragma unroll
-                for (int k = 0; k < V; ++k) {
-                    const int r = (k >> 1) * (2 * NT) + 2 * tid + (k & 1);
-                    const bool in = (r >= pos) && (r < pos + K);
-                    const bool ok = in && ((raw[k] & mask) <= (uint32_t)i_cur);
-                    inmask |= (in ? 1u : 0u) << k;
-                    fmask |= (ok ? 1u : 0u) << k;
-                }
-                // ---- early loads (branch free): own range cooperatively (x = tid + m*NT), targets of all candidates ----
-                LT vt[V], vj[V];
-#pragma unroll
-                for (int m = 0; m < V; ++m) {
-                    const int x = tid + m * NT;
-                    const bool ld = x < K;  // K <= i_cur / 4: never below the segment start
-                    vt[m] = ld ? ld_cs<LT>(a + base + (i_cur - (ld ? x : 0))) : (LT)0;
-                }
-#pragma unroll
-                for (int k = 0; k < V; ++k) {
-                    const bool ld = (fmask >> k) & 1u;
-                    vj[k] = ld ? ld_cg<LT>(a + base + (int64_t)(ld ? (raw[k] & mask) : 0u)) : (LT)0;
-                }
-                // ---- acceptance fixed point; c(k) = cb[k>>1] + (k odd ? bit(k-1) : 0); one barrier per iteration ----
-                int cb[R];
-                int total = 0;
-                uint32_t blo[R], bhi[R];
-                int buf = 0;
-#pragma unroll
-                for (int q = 0; q < R; ++q) {
-                    blo[q] = __ballot_sync(0xffffffffu, (fmask >> (2 * q)) & 1u);
-                    bhi[q] = __ballot_sync(0xffffffffu, (fmask >> (2 * q + 1)) & 1u);
-                    if (lane == 0) s_wsum[q * 32 + warp] = __popc(blo[q]) + __popc(bhi[q]);
-                }
-                int last_stamp = -1;  // stamp of the previous iteration of THIS window
-                while (true) {
-                    SQB_CONVERGE();
-                    __syncthreads();
-                    // the previous iteration changed nothing anywhere: fmask and the cb computed from it are final
-                    if (last_stamp >= 0 && s_misc[1] < last_stamp) break;
-                    const int* ws = s_wsum + buf * (R * 32);
-                    int run = 0;
-#pragma unroll
-                    for (int q = 0; q < R; ++q) {
-                        const int v = (lane < NW) ? ws[q * 32 + lane] : 0;
-                        int incl = v;
-#pragma unroll
-                        for (int d = 1; d < 32; d <<= 1) {
-                            const int t = __shfl_up_sync(0xffffffffu, incl, d);
-                            if (lane >= d) incl += t;
-                        }
-                        const int woff = __shfl_sync(0xffffffffu, incl - v, warp);
-                        const int tot = __shfl_sync(0xffffffffu, incl, 31);
-                        cb[q] = run + woff + __popc(blo[q] & lt_mask) + __popc(bhi[q] & lt_mask);
-                        run += tot;
-                    }
-                    total = run;
-                    uint32_t nf = 0;
-#pragma unroll
-                    for (int k = 0; k < V; ++k) {
-                        const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                        const uint32_t uk = raw[k] & mask;
-                        const bool ok = ((inmask >> k) & 1u) && uk <= (uint32_t)i_cur && (int)uk <= i_cur - ck;
-                        nf |= (ok ? 1u : 0u) << k;
-                    }
-                    ++stamp;
-                    last_stamp = stamp;
-                    if (nf != fmask) s_misc[1] = stamp;
-                    fmask = nf;
-                    buf ^= 1;
-                    int* wn = s_wsum + buf * (R * 32);
-#pragma unroll
-                    for (int q = 0; q < R; ++q) {
-                        blo[q] = __ballot_sync(0xffffffffu, (fmask >> (2 * q)) & 1u);
-                        bhi[q] = __ballot_sync(0xffffffffu, (fmask >> (2 * q + 1)) & 1u);
-                        if (lane == 0) wn[q * 32 + warp] = __popc(blo[q]) + __popc(bhi[q]);
-                    }
-                }
-                const bool phase_ends = total >= n_ph;
-                const int S = phase_ends ? n_ph : total;
-                const int own_lo = i_cur - S;
-                // ---- B: stage the original own-range values, build the target lists ----
-#pragma unroll
-                for (int m = 0; m < V; ++m) {
-                    const int x = tid + m * NT;
-                    if (x < S) s_otop[x] = vt[m];
-                }
-                uint32_t live = 0, ownm = 0;  // bit k: value k is step ck < S / its target lies in the window's own range
-                uint32_t slotv[V];
-#pragma unroll
-                for (int k = 0; k < V; ++k) slotv[k] = 0;
-#pragma unroll
-                for (int k = 0; k < V; ++k) {
-                    const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                    if (((fmask >> k) & 1u) && ck < S) {
-                        live |= 1u << k;
-                        if (phase_ends && ck == S - 1) s_misc[0] = (k >> 1) * (2 * NT) + 2 * tid + (k & 1);
-                        const uint32_t j = raw[k] & mask;
-                        if ((int)j > own_lo) {
-                            ownm |= 1u << k;
-                            const int u = i_cur - (int)j;  // u >= ck
-                            if (u != ck) {
-                                const uint32_t prev = atomicExch(&s_ohead[u], (uint32_t)ck);
-                                s_next[ck] = (uint16_t)prev;  // NONE32 truncates to NONE16
-                            }
-                        } else {
-                            uint32_t h = (j * 2654435761u) >> HS_SHIFT;
-                            const unsigned long long mine = ((unsigned long long)j << 32) | (unsigned)ck;
-                            uint32_t nxt = SQB_NONE16;
-                            while (true) {
-                                const unsigned long long prev = atomicCAS(&s_tab[h], SQB_EMPTY64, mine);
-                                if (prev == SQB_EMPTY64) break;
-                                if ((uint32_t)(prev >> 32) == j) {  // same target: push in front of the current head
-                                    if (atomicCAS(&s_tab[h], prev, mine) == prev) {
-                                        nxt = (uint32_t)prev & 0xFFFFu;
-                                        break;
-                                    }
-                                    continue;  // head moved, retry this slot
-                                }
-                                h = (h + 1) & (HS - 1);
-                            }
-                            s_next[ck] = (uint16_t)nxt;
-                            slotv[k] = h;
-                        }
-                    }
-                }
-                SQB_CONVERGE();
-                __syncthreads();
-                const int newpos = phase_ends ? (s_misc[0] + 1) : (pos + K);
-                // ---- C: every step resolves what it writes from the (now immutable) lists ----
-#pragma unroll
-                for (int k = 0; k < V; ++k) {
-                    if ((live >> k) & 1u) {
-                        const int ck = cb[k >> 1] + ((k & 1) ? (int)((fmask >> (k - 1)) & 1u) : 0);
-                        const uint32_t j = raw[k] & mask;
-                        LT val;
-                        if ((ownm >> k) & 1u) {
-                            const int u = i_cur - (int)j;
-                            if (u == ck) {
-                                val = sqb_list_T<LT>(s_ohead, s_next, s_otop, ck);
-                            } else {
-                                int mx;
-                                const int p = sqb_list_latest_before(s_next, s_ohead[u], ck, &mx);
-                                val = (p >= 0) ? sqb_list_T<LT>(s_ohead, s_next, s_otop, p) : s_otop[u];
-                            }
-                        } else {
-                            const uint32_t head = (uint32_t)s_tab[slotv[k]] & 0xFFFFu;
-                            int mx;
-                            const int p = sqb_list_latest_before(s_next, head, ck, &mx);
-                            val = (p >= 0) ? sqb_list_T<LT>(s_ohead, s_next, s_otop, p) : vj[k];
-                            if (mx == ck) a[base + (int64_t)j] = sqb_list_T<LT>(s_ohead, s_next, s_otop, ck);
-                        }
-                        st_cs<LT>(a + base + (i_cur - ck), val);  // final position: never read again by this kernel
-                    }
-                }
-                SQB_CONVERGE();
-                __syncthreads();
-                // ---- reset the list heads this thread pushed on (the next window's first barrier orders them) ----
-#pragma unroll
-                for (int k = 0; k < V; ++k) {
-                    const bool lv = (live >> k) & 1u, ow = (ownm >> k) & 1u;
-                    const uint32_t j = raw[k] & mask;
-                    if (lv && ow) s_ohead[i_cur - (int)j] = SQB_NONE32;
-                    if (lv && !ow) s_tab[slotv[k]] = SQB_EMPTY64;
-                }
-                i_cur -= S;
-                pos = newpos;
-            }
-        }
-    }
-}
-
-#endif  // SQB_TEST_VARIANTS
-#ifdef SQB_TEST_VARIANTS  // superseded replay variant: compiled into the test build only (tests/native/libsquidpy_b200_testvariants.so)
 // ------------------------------------------------------------------------------------------------
-// 2e. TWO-WARP PIPELINE per permutation.  ncu: 2c spends ~9 500 cycles per 192-step window in ONE dependent chain
-//     (PCG64 multiply-adds -> ballots/prefix -> hash inserts -> global loads -> stores) at IPC ~0.12, with HBM and the
-//     issue slots mostly idle.  The first half of that chain (RNG + rejection sampling) depends on nothing but the
-//     generator, so it is split off: the PRODUCER warp turns the PCG64 stream into lists of swap targets (one list
-//     per window) in a shared-memory ring, the CONSUMER warp applies the swaps of one window while the producer is
-//     already several windows ahead.  Hand-off with sequence counters in shared memory (one writer each).
-// ------------------------------------------------------------------------------------------------
-#define PIPE_RAW 256     // raw values per batch (Q = 4 outputs per lane)
-#define PIPE_NSLOT 4     // ring depth
-#define PIPE_HS 1024     // hash slots per team
-#define PIPE_TEAMS 2     // teams (producer + consumer warp) per CTA
-
-struct PipeSlot {
-    int S;         // number of steps; -1 = end of permutation
-    int i_cur;     // step s swaps positions base + i_cur - s and base + j[s]
-    long long base;
-    uint32_t j[PIPE_RAW];
-};
-
-template <typename LT>
-__global__ void __launch_bounds__(PIPE_TEAMS * 64) nhood_shuffle_pipe_kernel(LT* __restrict__ labels, int64_t stride,
-                                                                             const uint64_t* __restrict__ states,
-                                                                             int64_t n_perms, int nseg,
-                                                                             const int64_t* __restrict__ seg_start,
-                                                                             const int64_t* __restrict__ seg_len,
-                                                                             float wfactor) {
-    constexpr int Q = 4, RAW = PIPE_RAW, HS = PIPE_HS, HS_SHIFT = 22;
-    __shared__ PipeSlot s_slot_all[PIPE_TEAMS][PIPE_NSLOT];
-    __shared__ unsigned long long s_tab_all[PIPE_TEAMS][HS];
-    __shared__ uint32_t s_flag_all[PIPE_TEAMS][RAW / 32];
-    __shared__ unsigned s_full_all[PIPE_TEAMS][PIPE_NSLOT], s_empty_all[PIPE_TEAMS][PIPE_NSLOT];
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int team = warp >> 1, role = warp & 1;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-    PipeSlot* slots = s_slot_all[team];
-    unsigned long long* s_tab = s_tab_all[team];
-    uint32_t* s_flag = s_flag_all[team];
-    volatile unsigned* s_full = s_full_all[team];
-    volatile unsigned* s_empty = s_empty_all[team];
-    if (role == 0) {
-        for (int h = lane; h < HS; h += 32) s_tab[h] = SQB_EMPTY64;
-        if (lane < RAW / 32) s_flag[lane] = 0;
-        if (lane < PIPE_NSLOT) {
-            s_full[lane] = 0;
-            s_empty[lane] = 0;
-        }
-    }
-    __syncthreads();
-
-    const int64_t teams_total = (int64_t)gridDim.x * PIPE_TEAMS;
-    const int64_t team_id = (int64_t)blockIdx.x * PIPE_TEAMS + team;
-    unsigned w = 0;  // window counter of this team (same sequence in both warps)
-
-    if (role == 0) {
-        // ================= PRODUCER: PCG64 stream -> per-window target lists =================
-        u128 M32, C32, Mt, Ct;
-        pcg_jump_consts(32, M32, C32);
-        pcg_jump_consts((uint64_t)lane + 1, Mt, Ct);
-        for (int64_t perm = team_id; perm < n_perms; perm += teams_total) {
-            const uint64_t* st4 = states + perm * 4;
-            const u128 inc = mk128(st4[2], st4[3]);
-            u128 st = Mt * mk128(st4[0], st4[1]) + Ct * inc;
-            const u128 C32_inc = C32 * inc;
-            uint32_t raw[2 * Q];
-#pragma unroll
-            for (int k = 0; k < 2 * Q; ++k) raw[k] = 0;
-            int pos = RAW;
-            for (int seg = 0; seg <= nseg; ++seg) {
-                const bool last = (seg == nseg);
-                const long long base = last ? 0 : seg_start[seg];
-                int i_cur = last ? 0 : (int)(seg_len[seg] - 1);
-                while (last || i_cur >= 1) {
-                    int S = -1, newpos = pos;
-                    uint32_t u[2 * Q];
-                    bool F[2 * Q];
-                    int c[2 * Q];
-#pragma unroll
-                    for (int k = 0; k < 2 * Q; ++k) {
-                        u[k] = 0;
-                        F[k] = false;
-                        c[k] = 0;
-                    }
-                    if (!last) {
-                        if (pos >= RAW) {
-#pragma unroll
-                            for (int q = 0; q < Q; ++q) {
-                                const uint64_t o = pcg_output(st);
-                                st = M32 * st + C32_inc;
-                                raw[2 * q] = (uint32_t)o;
-                                raw[2 * q + 1] = (uint32_t)(o >> 32);
-                            }
-                            pos = 0;
-                        }
-                        const uint32_t mask = 0xFFFFFFFFu >> __clz(i_cur);
-                        const int i_lo = (int)(mask >> 1) + 1;
-                        const int n_ph = i_cur - i_lo + 1;
-                        const int K = sqb_window_size((int64_t)i_cur, RAW - pos, RAW, wfactor);
-                        bool inw[2 * Q];
-#pragma unroll
-                        for (int k = 0; k < 2 * Q; ++k) {
-                            const int r = (k >> 1) * 64 + 2 * lane + (k & 1);
-                            inw[k] = (r >= pos) && (r < pos + K);
-                            u[k] = raw[k] & mask;
-                            F[k] = inw[k] && (u[k] <= (uint32_t)i_cur);
-                        }
-                        int total = 0;
-                        while (true) {
-                            int run = 0;
-#pragma unroll
-                            for (int q = 0; q < Q; ++q) {
-                                const uint32_t blo = __ballot_sync(0xffffffffu, F[2 * q]);
-                                const uint32_t bhi = __ballot_sync(0xffffffffu, F[2 * q + 1]);
-                                c[2 * q] = run + __popc(blo & lt_mask) + __popc(bhi & lt_mask);
-                                c[2 * q + 1] = c[2 * q] + (F[2 * q] ? 1 : 0);
-                                run += __popc(blo) + __popc(bhi);
-                            }
-                            total = run;
-                            bool changed = false;
-#pragma unroll
-                            for (int k = 0; k < 2 * Q; ++k) {
-                                const bool nf = inw[k] && ((int)u[k] <= i_cur - c[k]) && (u[k] <= (uint32_t)i_cur);
-                                changed |= (nf != F[k]);
-                                F[k] = nf;
-                            }
-                            if (!__any_sync(0xffffffffu, changed)) break;
-                        }
-                        if (total >= n_ph) {
-                            S = n_ph;
-                            int myr = -1;
-#pragma unroll
-                            for (int k = 0; k < 2 * Q; ++k)
-                                if (F[k] && c[k] == S - 1) myr = (k >> 1) * 64 + 2 * lane + (k & 1);
-                            const uint32_t who = __ballot_sync(0xffffffffu, myr >= 0);
-                            newpos = __shfl_sync(0xffffffffu, myr, __ffs(who) - 1) + 1;
-                        } else {
-                            S = total;
-                            newpos = pos + K;
-                        }
-                    }
-                    if (last || S > 0) {
-                        // hand the window over: wait for the ring slot, fill it, publish
-                        const int slot = (int)(w % PIPE_NSLOT);
-                        const unsigned gen = w / PIPE_NSLOT;
-                        if (lane == 0)
-                            while (s_empty[slot] != gen) __nanosleep(64);
-                        __syncwarp();
-                        PipeSlot* sl = &slots[slot];
-#pragma unroll
-                        for (int k = 0; k < 2 * Q; ++k)
-                            if (F[k] && c[k] < S) sl->j[c[k]] = u[k];
-                        if (lane == 0) {
-                            sl->S = S;
-                            sl->i_cur = i_cur;
-                            sl->base = base;
-                        }
-                        __threadfence_block();
-                        __syncwarp();
-                        if (lane == 0) s_full[slot] = gen + 1;
-                        ++w;
-                    }
-                    if (last) break;
-                    i_cur -= S;
-                    pos = newpos;
-                }
-            }
-        }
-    } else {
-        // ================= CONSUMER: apply the swaps of one window at a time =================
-        for (int64_t perm = team_id; perm < n_perms; perm += teams_total) {
-            LT* __restrict__ a = labels + perm * stride;
-            while (true) {
-                const int slot = (int)(w % PIPE_NSLOT);
-                const unsigned gen = w / PIPE_NSLOT;
-                if (lane == 0)
-                    while (s_full[slot] != gen + 1) __nanosleep(32);
-                __syncwarp();
-                const PipeSlot* sl = &slots[slot];
-                const int S = sl->S;
-                const int i_cur = sl->i_cur;
-                const long long base = sl->base;
-                if (S > 0) {
-                    const int own_lo = i_cur - S;
-                    uint32_t jv[2 * Q];
-                    uint32_t actm = 0, insm = 0;
-                    int slotv[2 * Q];
-#pragma unroll
-                    for (int t = 0; t < 2 * Q; ++t) {
-                        const int s = lane + 32 * t;
-                        jv[t] = 0;
-                        slotv[t] = 0;
-                        if (s < S) {
-                            const uint32_t j = sl->j[s];
-                            jv[t] = j;
-                            if ((int)j > own_lo) {
-                                const int s2 = i_cur - (int)j;
-                                if (s2 != s) {
-                                    actm |= 1u << t;
-                                    atomicOr(&s_flag[s >> 5], 1u << (s & 31));
-                                    atomicOr(&s_flag[s2 >> 5], 1u << (s2 & 31));
-                                }
-                            } else {
-                                actm |= 1u << t;
-                                uint32_t h = (j * 2654435761u) >> HS_SHIFT;
-                                const unsigned long long mine = ((unsigned long long)j << 32) | (unsigned)s;
-                                while (true) {
-                                    const unsigned long long prev = atomicCAS(&s_tab[h], SQB_EMPTY64, mine);
-                                    if (prev == SQB_EMPTY64) {
-                                        insm |= 1u << t;
-                                        slotv[t] = (int)h;
-                                        break;
-                                    }
-                                    if ((uint32_t)(prev >> 32) == j) {
-                                        const int so = (int)(uint32_t)prev;
-                                        atomicOr(&s_flag[s >> 5], 1u << (s & 31));
-                                        atomicOr(&s_flag[so >> 5], 1u << (so & 31));
-                                        break;
-                                    }
-                                    h = (h + 1) & (HS - 1);
-                                }
-                            }
-                        }
-                    }
-                    __syncwarp();
-                    // conflict-free swaps straight on global memory: all loads, then all stores (branch-free)
-                    LT vi[2 * Q], vj[2 * Q];
-                    uint32_t dirm = 0;
-#pragma unroll
-                    for (int t = 0; t < 2 * Q; ++t) {
-                        const int s = lane + 32 * t;
-                        const bool act = (actm >> t) & 1u;
-                        const int ss = act ? s : 0;
-                        const bool dir = act && !((s_flag[ss >> 5] >> (ss & 31)) & 1u);
-                        dirm |= (dir ? 1u : 0u) << t;
-                        vi[t] = dir ? ld_cs<LT>(a + base + (i_cur - ss)) : (LT)0;
-                        vj[t] = dir ? ld_cg<LT>(a + base + (long long)jv[t]) : (LT)0;
-                    }
-#pragma unroll
-                    for (int t = 0; t < 2 * Q; ++t) {
-                        const int s = lane + 32 * t;
-                        const bool dir = (dirm >> t) & 1u;
-                        const int ss = dir ? s : 0;
-                        if (dir) st_cs<LT>(a + base + (i_cur - ss), vj[t]);  // final: evict first
-                        if (dir) a[base + (long long)jv[t]] = vi[t];
-                    }
-                    // conflicting swaps in step order (disjoint from the set above), lane 0, on global memory
-                    const uint32_t fw = (lane < RAW / 32) ? s_flag[lane] : 0u;
-                    if (__ballot_sync(0xffffffffu, fw != 0u)) {
-                        if (lane == 0) {
-                            for (int wd = 0; wd < RAW / 32; ++wd) {
-                                uint32_t bits = s_flag[wd];
-                                while (bits) {
-                                    const int b = __ffs(bits) - 1;
-                                    bits &= bits - 1;
-                                    const int s = wd * 32 + b;
-                                    const long long pi = base + (i_cur - s), pj = base + (long long)sl->j[s];
-                                    const LT x = ld_cg<LT>(a + pi), y = ld_cg<LT>(a + pj);
-                                    a[pi] = y;
-                                    a[pj] = x;
-                                }
-                            }
-                        }
-                        __syncwarp();
-                        if (lane < RAW / 32) s_flag[lane] = 0;
-                    }
-#pragma unroll
-                    for (int t = 0; t < 2 * Q; ++t)
-                        if ((insm >> t) & 1u) s_tab[slotv[t]] = SQB_EMPTY64;
-                }
-                // release the slot (also orders this window's global stores before the next window's loads)
-                __threadfence_block();
-                __syncwarp();
-                if (lane == 0) s_empty[slot] = gen + 1;
-                ++w;
-                if (S < 0) break;  // end of this permutation
-            }
-        }
-    }
-}
-
-#endif  // SQB_TEST_VARIANTS
-// ------------------------------------------------------------------------------------------------
-// 2f. TWO-KERNEL replay (algo 5).  ncu showed every fused variant to be bound by random DRAM row activations (1000
-//     live 1 MB label arrays do not fit the 126 MB L2) and, with fewer permutations in flight, by the dependent
-//     instruction chain RNG -> rejection -> swaps.  Splitting the replay removes both:
-//       nhood_jgen_kernel   one warp per permutation, ALL permutations in flight (pure ALU + ballots, no random
-//                           memory traffic): replays PCG64 + masked rejection and streams the Fisher-Yates target
-//                           of every step i to J[perm][i] (coalesced 4-byte stores, read once, evict-first);
-//       nhood_apply_kernel  one CTA per permutation, few permutations in flight (label arrays stay L2 resident):
-//                           takes S consecutive steps per window (no RNG, no prefix sums: the targets are already
-//                           known), detects position sharing (own-range targets, duplicate targets via a
-//                           shared-memory hash table), swaps conflict-free steps straight in global memory and
-//                           replays the few conflicting ones in step order on staged copies.
+// 2d. Swap-target generation, the first half of the TWO-KERNEL replay (shuffle_algo 7).  ncu showed the one-kernel
+//     replays (2a, 2b) to be bound by random DRAM row activations (1000 live 1 MB label arrays do not fit the 126 MB L2)
+//     and, with fewer permutations in flight, by the dependent instruction chain RNG -> rejection -> swaps.  Splitting
+//     the replay removes both:
+//       nhood_jgen_kernel        one warp per permutation, ALL permutations in flight (pure ALU + ballots, no random
+//                                memory traffic): replays PCG64 + masked rejection and streams the Fisher-Yates target
+//                                of every step i to J[perm][i] (coalesced 4-byte stores, read once, evict-first);
+//       nhood_apply_list_kernel  one CTA per permutation, few permutations in flight, applies the swaps (2e).
 // ------------------------------------------------------------------------------------------------
 template <int Q>
 __global__ void __launch_bounds__(128) nhood_jgen_kernel(uint32_t* __restrict__ J, int64_t stride,
@@ -1637,219 +752,16 @@ __global__ void __launch_bounds__(128) nhood_jgen_kernel(uint32_t* __restrict__ 
     }
 }
 
-#ifdef SQB_TEST_VARIANTS  // superseded replay variant: compiled into the test build only (tests/native/libsquidpy_b200_testvariants.so)
-template <typename LT, int NT, int SPT>
-__global__ void __launch_bounds__(NT) nhood_apply_kernel(LT* __restrict__ labels, const uint32_t* __restrict__ J,
-                                                         int64_t stride, int64_t n_perms, int nseg,
-                                                         const int64_t* __restrict__ seg_start,
-                                                         const int64_t* __restrict__ seg_len, float wfactor, int low_cap,
-                                                         uint64_t stagger_ns) {
-    // low_cap > 0: positions [0, min(low_cap, segment length)) of the current segment live in shared memory for the
-    // whole replay.  Targets are uniform in [0, i], so with 176 KB about half of all random accesses of a 1M-element
-    // shuffle never leave the SM (ncu: the kernel is bound by the ~1.8 cycles/request the LSU needs for uncoalesced
-    // global accesses; shared memory serves a whole warp of random bytes in a few cycles).
-    constexpr int W = NT * SPT;  // max steps per window
-    constexpr int HS = 2 * W;
-    constexpr int LOG_HS = (HS == 1024 ? 10 : HS == 2048 ? 11 : HS == 4096 ? 12 : HS == 8192 ? 13 : 14);
-    static_assert(HS == (1 << LOG_HS), "HS");
-    constexpr int HS_SHIFT = 32 - LOG_HS;
-    extern __shared__ __align__(16) unsigned char sqb_shuffle_smem[];
-    unsigned long long* s_tab = reinterpret_cast<unsigned long long*>(sqb_shuffle_smem);
-    uint32_t* s_sj = reinterpret_cast<uint32_t*>(s_tab + HS);
-    uint32_t* s_flag = s_sj + W;
-    int* s_misc = reinterpret_cast<int*>(s_flag + W / 32);
-    LT* s_own = reinterpret_cast<LT*>(s_misc + 4);
-    LT* s_hval = s_own + W;
-    LT* s_low = s_hval + HS;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    for (int h = tid; h < HS; h += NT) s_tab[h] = SQB_EMPTY64;
-    for (int w = tid; w < W / 32; w += NT) s_flag[w] = 0;
-    if (tid < 4) s_misc[tid] = 0;
-    sqb_stagger(stagger_ns * blockIdx.x / gridDim.x);
-    __syncthreads();
-
-    for (int64_t perm = blockIdx.x; perm < n_perms; perm += gridDim.x) {
-        LT* __restrict__ a = labels + perm * stride;
-        const uint32_t* __restrict__ Jp = J + perm * stride;
-        for (int seg = 0; seg < nseg; ++seg) {
-            const int64_t base = seg_start[seg];
-            int i_cur = (int)(seg_len[seg] - 1);
-            const int low_n = (int)(seg_len[seg] < (int64_t)low_cap ? seg_len[seg] : (int64_t)low_cap);
-            for (int p = tid; p < low_n; p += NT) s_low[p] = a[base + p];
-            __syncthreads();
-            while (i_cur >= 1) {
-                // window: steps i_cur, i_cur-1, ..., i_cur-S+1 (all >= 1); ~constant expected number of conflicts
-                int S = (int)(wfactor * sqrtf((float)i_cur));
-                S = S < 32 ? 32 : S;
-                S = S > W ? W : S;
-                S = S > i_cur ? i_cur : S;
-                const int own_lo = i_cur - S;
-                uint32_t jv[SPT], slotv[SPT];
-                uint32_t actm = 0, insm = 0;
-                // ---- phase 1: targets (coalesced, streaming), own-range check, hash insert ----
-#pragma unroll
-                for (int k = 0; k < SPT; ++k) {
-                    const int s = tid + k * NT;
-                    const bool live = s < S;
-                    const uint32_t j = live ? __ldcs(Jp + base + (i_cur - (live ? s : 0))) : 0u;
-                    jv[k] = j;
-                    slotv[k] = 0;
-                    if (live) s_sj[s] = j;
-                }
-#pragma unroll
-                for (int k = 0; k < SPT; ++k) {
-                    const int s = tid + k * NT;
-                    if (s < S) {
-                        const uint32_t j = jv[k];
-                        if ((int)j > own_lo) {
-                            const int s2 = i_cur - (int)j;
-                            if (s2 != s) {
-                                actm |= 1u << k;
-                                atomicOr(&s_flag[s >> 5], 1u << (s & 31));
-                                atomicOr(&s_flag[s2 >> 5], 1u << (s2 & 31));
-                            }
-                        } else {
-                            actm |= 1u << k;
-                            uint32_t h = (j * 2654435761u) >> HS_SHIFT;
-                            const unsigned long long mine = ((unsigned long long)j << 32) | (unsigned)s;
-                            while (true) {
-                                const unsigned long long prev = atomicCAS(&s_tab[h], SQB_EMPTY64, mine);
-                                if (prev == SQB_EMPTY64) {
-                                    insm |= 1u << k;
-                                    slotv[k] = h;
-                                    break;
-                                }
-                                if ((uint32_t)(prev >> 32) == j) {
-                                    const int so = (int)(uint32_t)prev;
-                                    atomicOr(&s_flag[s >> 5], 1u << (s & 31));
-                                    atomicOr(&s_flag[so >> 5], 1u << (so & 31));
-                                    break;
-                                }
-                                h = (h + 1) & (HS - 1);
-                            }
-                        }
-                    }
-                }
-                SQB_CONVERGE_W();
-                __syncthreads();
-                // ---- phase 2 (branch-free): conflict-free swaps in global memory, conflicting steps staged ----
-                uint32_t dirm = 0, stgm = 0;
-                {
-                    LT vi[SPT], vj[SPT];
-#pragma unroll
-                    for (int k = 0; k < SPT; ++k) {
-                        const int s = tid + k * NT;
-                        const bool live = s < S;
-                        const int ss = live ? s : 0;
-                        const bool flagged = live && ((s_flag[ss >> 5] >> (ss & 31)) & 1u);
-                        const bool dir = live && !flagged && ((actm >> k) & 1u);
-                        const bool ins = (insm >> k) & 1u;
-                        stgm |= (flagged ? 1u : 0u) << k;
-                        dirm |= (dir ? 1u : 0u) << k;
-                        const bool ldt = dir || (flagged && ins);
-                        const bool ldo = dir || flagged;
-                        const int po = i_cur - ss;              // own position (segment relative)
-                        const int pt = (int)(ldt ? jv[k] : 0u);  // target position
-                        LT xo = (LT)0, xt = (LT)0;
-                        if (ldo && po < low_n) xo = s_low[po];
-                        if (ldo && po >= low_n) xo = ld_cs<LT>(a + base + po);
-                        if (ldt && pt < low_n) xt = s_low[pt];
-                        if (ldt && pt >= low_n) xt = ld_cg<LT>(a + base + pt);
-                        vi[k] = xo;
-                        vj[k] = xt;
-                    }
-#pragma unroll
-                    for (int k = 0; k < SPT; ++k) {
-                        const int s = tid + k * NT;
-                        const bool dir = (dirm >> k) & 1u, stg = (stgm >> k) & 1u, ins = (insm >> k) & 1u;
-                        const int ss = (dir || stg) ? s : 0;
-                        const int po = i_cur - ss, pt = (int)jv[k];
-                        if (dir && po < low_n) s_low[po] = vj[k];
-                        if (dir && po >= low_n) st_cs<LT>(a + base + po, vj[k]);
-                        if (dir && pt < low_n) s_low[pt] = vi[k];
-                        if (dir && pt >= low_n) a[base + pt] = vi[k];
-                        if (stg) s_own[ss] = vi[k];
-                        if (stg && ins) s_hval[slotv[k]] = vj[k];
-                    }
-                }
-                if (stgm) s_misc[1] = 1;
-                SQB_CONVERGE_W();
-                __syncthreads();
-                const int any_flag = s_misc[1];
-                if (any_flag) {
-                    // ---- phase 3: ordered replay of the conflicting steps on the staged values ----
-                    if (warp == 0) {
-                        const int nwords = (S + 31) >> 5;
-                        for (int wb = 0; wb < nwords; wb += 32) {
-                            const uint32_t myw = (wb + lane < nwords) ? s_flag[wb + lane] : 0u;
-                            uint32_t nz = __ballot_sync(0xffffffffu, myw != 0u);
-                            while (nz) {
-                                const int wl = __ffs(nz) - 1;
-                                nz &= nz - 1;
-                                uint32_t bits = __shfl_sync(0xffffffffu, myw, wl);
-                                if (lane == 0) {
-                                    while (bits) {
-                                        const int b = __ffs(bits) - 1;
-                                        bits &= bits - 1;
-                                        const int s = (wb + wl) * 32 + b;
-                                        const uint32_t j = s_sj[s];
-                                        const LT x = s_own[s];
-                                        if ((int)j > own_lo) {
-                                            const int s2 = i_cur - (int)j;
-                                            if (s2 != s) {
-                                                const LT y = s_own[s2];
-                                                s_own[s] = y;
-                                                s_own[s2] = x;
-                                            }
-                                        } else {
-                                            uint32_t h = (j * 2654435761u) >> HS_SHIFT;
-                                            while ((uint32_t)(s_tab[h] >> 32) != j) h = (h + 1) & (HS - 1);
-                                            const LT y = s_hval[h];
-                                            s_own[s] = y;
-                                            s_hval[h] = x;
-                                        }
-                                    }
-                                }
-                            }
-                        }
-                    }
-                    __syncthreads();
-#pragma unroll
-                    for (int k = 0; k < SPT; ++k) {
-                        const int s = tid + k * NT;
-                        const bool stg = (stgm >> k) & 1u, ins = (insm >> k) & 1u;
-                        const int ss = stg ? s : 0;
-                        const int po = i_cur - ss, pt = (int)jv[k];
-                        if (stg && po < low_n) s_low[po] = s_own[ss];
-                        if (stg && po >= low_n) st_cs<LT>(a + base + po, s_own[ss]);
-                        if (stg && ins && pt < low_n) s_low[pt] = s_hval[slotv[k]];
-                        if (stg && ins && pt >= low_n) a[base + pt] = s_hval[slotv[k]];
-                    }
-                    __syncthreads();
-                    for (int w = tid; w < ((S + 31) >> 5); w += NT) s_flag[w] = 0;
-                    if (tid == 0) s_misc[1] = 0;
-                }
-#pragma unroll
-                for (int k = 0; k < SPT; ++k)
-                    if ((insm >> k) & 1u) s_tab[slotv[k]] = SQB_EMPTY64;
-                __syncthreads();
-                i_cur -= S;
-            }
-            // segment done: the shared-memory resident low part goes back to global memory
-            for (int p = tid; p < low_n; p += NT) a[base + p] = s_low[p];
-            __syncthreads();
-        }
-    }
-}
-
-#endif  // SQB_TEST_VARIANTS
 // ------------------------------------------------------------------------------------------------
-// 2h. TWO-KERNEL replay with list-based conflict resolution (shuffle_algo 7): nhood_jgen_kernel (2f, a warp per
+// 2e. TWO-KERNEL replay with list-based conflict resolution (shuffle_algo 7): nhood_jgen_kernel (2d, a warp per
 //     permutation, warp-level synchronisation only) turns the PCG64 streams into the swap targets J[perm][i]; this kernel
-//     applies them, one CTA per permutation, W = NT*SPT Fisher-Yates steps per window.  Step s of a window (top position
-//     i_cur - s) belongs to thread s % NT: the J values, the own range and its write-back are fully coalesced, no ranks,
-//     ballots or acceptance barriers are left in this kernel, and conflicts are resolved exactly as in 2g (per-position
-//     lists, original values only, no ordered pass).  The next window's J values are prefetched into registers.
+//     applies them, one CTA per permutation, W = NT*SPT Fisher-Yates steps per window.  Few permutations are in flight:
+//     measured on B200 (tools/micro/rmw_bench.cu), random byte swaps over label arrays that stay inside the 126 MB L2
+//     run at ~55 G swaps/s, over 1000 arrays (1 GB) at ~20 G swaps/s, because every swap then costs two random 32-byte
+//     DRAM sectors.  Step s of a window (top position i_cur - s) belongs to thread s % NT: the J values, the own range
+//     and its write-back are fully coalesced, no ranks, ballots or acceptance barriers are left in this kernel, and
+//     conflicts are resolved as in 2c (per-position lists, original values only, no ordered pass).  The next window's J
+//     values are prefetched into registers.
 //     ncu on the first version (every outside target inserted into the hash table): 43% of all instructions and most
 //     short-scoreboard stalls were the dependent 64-bit CAS probe chains, and the barrier stalls (25%) their imbalance.
 //     Duplicate targets are rare, so they are now FILTERED first: two bits per bucket (bucket = target mod 32W) in shared
@@ -2035,7 +947,7 @@ __global__ void __launch_bounds__(NT, 1) nhood_apply_list_kernel(LT* __restrict_
                 }
                 SQB_CONVERGE();
                 __syncthreads();
-                // ---- C: every step derives what it writes from the (now immutable) lists, original values only (2g) ----
+                // ---- C: every step derives what it writes from the (now immutable) lists, original values only (2c) ----
 #pragma unroll
                 for (int m = 0; m < SPT; ++m) {
                     const int s = tid + m * NT;
@@ -2104,440 +1016,6 @@ __global__ void __launch_bounds__(NT, 1) nhood_apply_list_kernel(LT* __restrict_
 }
 
 // ------------------------------------------------------------------------------------------------
-// 2i. REGION replay (shuffle_algo 8; compiled into the TEST build only, like the other superseded variants): the apply step of
-//     the two-kernel replay with EVERY random access in shared memory.  Measured at 1M spots x 1000 permutations: 22.9 ms against
-//     16.0 ms for the list kernel 2h -- with the memory system out of the way the replay is bound by instruction issue
-//     (17 G warp instructions: the J row is re-scanned (R+1)/2 = 4 times, and every window pays for compaction, filter and
-//     three block barriers), see DESIGN.md 3.1.  Kept as an independent cross-check of 2h: a different decomposition of the
-//     same Fisher-Yates sweep that must produce the same permutations.
-//     tools/micro/smem_bench.cu on B200: a random byte read + write costs 5.3 cycles per warp in the CTA's own shared
-//     memory, 135 in distributed shared memory of a cluster and 230 against an L2-resident global array -- the list kernel
-//     (2h) spends most of its time on the two thirds of its targets that miss its shared-memory low part.  A 1 MB label
-//     array does not fit one SM, but Fisher-Yates only ever exchanges a top i with a target j <= i, so the array can be
-//     processed one REGION [lo, hi) of <= ~165 K positions at a time, top region first, every step exactly once, in the
-//     pass of the region its TARGET falls into:
-//       pass of region r:  slab <- a[lo, hi)                                                  (coalesced)
-//         scan the steps i = m-1 .. max(lo, 1) (J row, coalesced, prefetched one chunk ahead); the steps whose target lies
-//         in [lo, hi) are compacted IN STEP ORDER into windows of <= W slots and applied: v = slab[j]; slab[j] = top;
-//         top = v, where the top is a[i] for a step above the region (a[i] still holds T(i), the value position i had just
-//         before step i: the pass of i's own region left it there and no pass in between touches it) or slab[i - lo] for a
-//         step inside it.  A step whose target lies BELOW the region is simply not in any window of this pass: whatever
-//         earlier steps deposited at its top stays there as T(i) for the pass that owns its target.
-//         a[lo, hi) <- slab                                                                    (coalesced)
-//     Conflicts inside a window are resolved as in 2g/2h from immutable lists and original values only (no ordered pass),
-//     now keyed by POSITION (tests/emu_shuffle.py::_resolve_general_window is the executable specification): targeters[p] =
-//     slots with target p, owner[p] = the slot whose top is p; T(x) = T(latest targeter of x's top) or its original value;
-//     slot s writes top_s <- T(latest earlier targeter of its target) or the target's original value; the last targeter of p
-//     deposits T(itself) at p unless p's owner is in the window.  Only positions whose filter bucket was marked twice (a few
-//     percent) touch the hash tables at all.
-//     Cost besides the resolution: the J row is re-scanned once per region above the target region, (R-1)/2 extra passes
-//     over J for R regions (streaming, 6 regions at 1M spots).
-// ------------------------------------------------------------------------------------------------
-#ifdef SQB_TEST_VARIANTS
-template <typename LT, int NT>
-__global__ void __launch_bounds__(NT, 1) nhood_apply_region_kernel(LT* __restrict__ labels, const uint32_t* __restrict__ J,
-                                                                   int64_t stride, int64_t n_perms, int nseg,
-                                                                   const int64_t* __restrict__ seg_start,
-                                                                   const int64_t* __restrict__ seg_len, uint32_t full_mask,
-                                                                   uint64_t stagger_ns, int region_cap) {
-    // Work distribution inside a window.  A chunk of NT*K consecutive steps is scanned, warp w takes the w-th run of 32*K of
-    // them: it compacts ITS matches in step order into its own segment of the slot arrays (ids w*CAPW + r: id order = step
-    // order) with nothing but ballots, and then processes them 32 at a time with full lanes.  Slots on multiply-marked
-    // positions (a few percent) are compacted once more per warp and resolved by lanes 0..n-1 of the warp in one pass per
-    // phase, so the list code never runs with one or two live lanes per iteration.  Three block barriers per window:
-    // filter marks complete / lists complete / writes complete.
-    constexpr int NWARP = NT / 32;
-    constexpr int KMAX = 16;          // J values scanned per thread and chunk, at most
-    constexpr int CAPW = 96;          // slot ids per warp
-    constexpr int ITMAX = CAPW / 32;  // dense iterations per warp and window, at most
-    constexpr int NID = NWARP * CAPW;
-    constexpr int HS = 2 * NT;        // slots per window, at most = hash slots per table
-    constexpr int NWB = 2 * HS;       // filter words (16 buckets of 2 bits each)
-    constexpr int QSH = 18;           // slot entry = (chunk offset << 18) | (target - lo)
-    constexpr int ETGT = 56;          // expected matches per warp a chunk is sized for (CAPW is 5 sigma above)
-    constexpr int LOG_HS = (HS == 512 ? 9 : HS == 1024 ? 10 : HS == 2048 ? 11 : HS == 4096 ? 12 : 13);
-    static_assert(HS == (1 << LOG_HS), "HS must be a power of two");
-    static_assert(NID < 0xFFFF, "slot ids are stored in 16 bits");
-    static_assert(NT * KMAX <= (1 << (32 - QSH)), "chunk offsets must fit the slot entry");
-    static_assert(NT * 2 <= HS && 64 <= CAPW, "two steps per thread must always fit a window");
-    constexpr int HS_SHIFT = 32 - LOG_HS;
-    extern __shared__ __align__(16) unsigned char sqb_shuffle_smem[];
-    unsigned long long* s_tabT = reinterpret_cast<unsigned long long*>(sqb_shuffle_smem);  // [HS] (position << 32) | head of its targeter list
-    unsigned long long* s_tabO = s_tabT + HS;                                              // [HS] (position << 32) | slot whose top it is
-    uint32_t* s_bits = reinterpret_cast<uint32_t*>(s_tabO + HS);                            // [NWB] duplicate filter
-    uint32_t* s_q = s_bits + NWB;                                                           // [NID] the window's slots
-    uint32_t* s_cnt = s_q + NID;                                                            // [64] slots per warp
-    uint16_t* s_next = reinterpret_cast<uint16_t*>(s_cnt + 64);                             // [NID] list links
-    uint16_t* s_slow = s_next + NID;                                                        // [NWARP][32] slots of multiply-marked positions
-    LT* s_otop = reinterpret_cast<LT*>(s_slow + NWARP * 32);                                // [NID] original top values
-    LT* s_slab = s_otop + NID;                                                              // [region_cap] the region
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-    for (int h = tid; h < 2 * HS; h += NT) s_tabT[h] = SQB_EMPTY64;  // both tables
-    for (int w = tid; w < NWB; w += NT) s_bits[w] = 0u;
-    sqb_stagger(stagger_ns * blockIdx.x / gridDim.x);
-    __syncthreads();
-
-    // duplicate filter: "marked" / "marked again" bits of the bucket of position pl (2h)
-    auto mark_pos = [&](uint32_t pl) {
-        const uint32_t sh = (pl & 15u) * 2u;
-        uint32_t* wp = &s_bits[(pl >> 4) & (NWB - 1)];
-        const uint32_t old = atomicOr(wp, 1u << sh);
-        if ((old >> sh) & 1u) atomicOr(wp, 2u << sh);
-    };
-    auto marked_again = [&](uint32_t pl) -> bool { return (s_bits[(pl >> 4) & (NWB - 1)] >> ((pl & 15u) * 2u + 1u)) & 1u; };
-    // push slot id on the targeter list of position pl; returns the table slot
-    auto push_targeter = [&](uint32_t pl, int id) -> uint32_t {
-        uint32_t h = (pl * 2654435761u) >> HS_SHIFT;
-        const unsigned long long mine = ((unsigned long long)pl << 32) | (unsigned)id;
-        uint32_t nxt = SQB_NONE16;
-        while (true) {
-            const unsigned long long prev = atomicCAS(&s_tabT[h], SQB_EMPTY64, mine);
-            if (prev == SQB_EMPTY64) break;
-            if ((uint32_t)(prev >> 32) == pl) {  // same position: push in front of the current head
-                if (atomicCAS(&s_tabT[h], prev, mine) == prev) {
-                    nxt = (uint32_t)prev & 0xFFFFu;
-                    break;
-                }
-                continue;
-            }
-            h = (h + 1) & (HS - 1);
-        }
-        s_next[id] = (uint16_t)nxt;
-        return h;
-    };
-    auto insert_owner = [&](uint32_t pl, int id) -> uint32_t {  // tops are distinct: plain insertion
-        uint32_t h = (pl * 2654435761u) >> HS_SHIFT;
-        const unsigned long long mine = ((unsigned long long)pl << 32) | (unsigned)id;
-        while (atomicCAS(&s_tabO[h], SQB_EMPTY64, mine) != SQB_EMPTY64) h = (h + 1) & (HS - 1);
-        return h;
-    };
-    auto find_key = [&](const unsigned long long* tab, uint32_t pl) -> int {  // table slot of position pl, or -1
-        uint32_t h = (pl * 2654435761u) >> HS_SHIFT;
-        for (int probes = 0; probes < HS; ++probes) {
-            const unsigned long long e = tab[h];
-            if (e == SQB_EMPTY64) return -1;
-            if ((uint32_t)(e >> 32) == pl) return (int)h;
-            h = (h + 1) & (HS - 1);
-        }
-        return -1;
-    };
-
-    for (int64_t perm = blockIdx.x; perm < n_perms; perm += gridDim.x) {
-        for (int seg = 0; seg < nseg; ++seg) {
-            const int64_t base = seg_start[seg];
-            const int m = (int)seg_len[seg];  // n < 2^31
-            if (m < 2) continue;
-            LT* __restrict__ a0 = labels + perm * stride + base;
-            const uint32_t* __restrict__ Jb = J + perm * stride + base;
-            const int R = (m + region_cap - 1) / region_cap;
-            const int B = (((m + R - 1) / R + 15) / 16) * 16;  // balanced regions, <= region_cap (a multiple of 16)
-            for (int r = (m - 1) / B; r >= 0; --r) {
-                const int lo = r * B;
-                const int len = min(B, m - lo);
-                const int hi = lo + len;
-                {  // slab <- a[lo, hi)
-                    const LT* __restrict__ src = a0 + lo;
-                    int x0 = 0;
-                    if ((reinterpret_cast<uintptr_t>(src) & 15u) == 0) {
-                        constexpr int EPV = 16 / (int)sizeof(LT);
-                        const int nv = len / EPV;
-                        const uint4* __restrict__ sv = reinterpret_cast<const uint4*>(src);
-                        uint4* dv = reinterpret_cast<uint4*>(s_slab);
-                        for (int x = tid; x < nv; x += NT) dv[x] = __ldcg(sv + x);
-                        x0 = nv * EPV;
-                    }
-                    for (int x = x0 + tid; x < len; x += NT) s_slab[x] = ld_cg<LT>(src + x);
-                }
-                __syncthreads();
-                const int i_min = max(lo, 1);
-                // chunk = NT*K consecutive steps from i_cur down, sized for ETGT expected matches per warp (two steps per thread
-                // always fit)
-                // (single precision is plenty: any block-uniform K is correct, this only sizes the windows).  K >= 4 is a multiple of
-                // 4: the scan then takes four consecutive J values per lane with one 16-byte load.
-                // (a first chunk of < 4 steps makes J[i_cur + 1] 16-byte aligned at every later chunk start: chunk lengths are
-                //  multiples of 4)
-                const int misalign = (int)((((uintptr_t)Jb >> 2) + (uintptr_t)m) & 3u);
-                constexpr bool vec_ok = true;
-                auto pick_k = [&](int i) -> int {
-                    const float num = (float)min(len, i - lo + 1);
-                    int k = (int)(((float)ETGT * ((float)i + 1.0f)) / (32.0f * num));
-                    k = k < 2 ? 2 : (k > KMAX ? KMAX : k);
-                    if (k >= 4) k &= ~3;
-                    return k;
-                };
-                // Scan layouts.  vector (K % 4 == 0 and vec_ok): step offset s = ((warp*K/4 + g)*32 + lane)*4 + e, jv[4g + e] = J[i_top - s]
-                // (one 16-byte load per g); scalar: s = (warp*K + k)*32 + lane, jv[k] = J[i_top - s].  Either way warp w scans the w-th
-                // run of 32*K steps and its (k, lane) resp. (g, lane, e) order is step order.
-                uint32_t jv[KMAX];
-                auto load_chunk = [&](int i_top, int K, int SC) {
-                    if ((K & 3) == 0 && vec_ok) {
-#pragma unroll
-                        for (int g = 0; g < KMAX / 4; ++g) {
-                            jv[4 * g] = jv[4 * g + 1] = jv[4 * g + 2] = jv[4 * g + 3] = 0u;
-                            if (4 * g < K) {  // block-uniform
-                                const int s0 = ((warp * (K >> 2) + g) * 32 + lane) * 4;
-                                if (s0 + 3 < SC) {
-                                    const uint4 v = __ldcs(reinterpret_cast<const uint4*>(Jb + (i_top - s0 - 3)));
-                                    jv[4 * g] = v.w, jv[4 * g + 1] = v.z, jv[4 * g + 2] = v.y, jv[4 * g + 3] = v.x;
-                                } else {
-#pragma unroll
-                                    for (int e = 0; e < 4; ++e)
-                                        if (s0 + e < SC) jv[4 * g + e] = __ldcs(Jb + (i_top - s0 - e));
-                                }
-                            }
-                        }
-                    } else {
-#pragma unroll
-                        for (int k = 0; k < KMAX; ++k) {
-                            jv[k] = 0u;
-                            if (k < K) {  // block-uniform
-                                const int s = (warp * K + k) * 32 + lane;
-                                if (s < SC) jv[k] = __ldcs(Jb + (i_top - s));
-                            }
-                        }
-                    }
-                };
-                int i_cur = m - 1;
-                int K = pick_k(i_cur);
-                int SC = min(NT * K, i_cur - i_min + 1);
-                if (misalign) K = 2, SC = min(misalign, SC);
-                load_chunk(i_cur, K, SC);
-                while (i_cur >= i_min) {
-                    // ---- S1: the warp compacts its matches, in step order, into its segment of the slot array ----
-                    const int idb = warp * CAPW;
-                    uint32_t cnt = 0;
-                    if ((K & 3) == 0 && vec_ok) {
-#pragma unroll
-                        for (int g = 0; g < KMAX / 4; ++g) {
-                            if (4 * g < K) {
-                                const int s0 = ((warp * (K >> 2) + g) * 32 + lane) * 4;
-                                uint32_t jl[4], bb[4];
-                                bool mt[4];
-#pragma unroll
-                                for (int e = 0; e < 4; ++e) {
-                                    jl[e] = jv[4 * g + e] - (uint32_t)lo;
-                                    mt[e] = (s0 + e < SC) && jl[e] < (uint32_t)len;
-                                    bb[e] = __ballot_sync(0xffffffffu, mt[e]);
-                                }
-                                // slots in (lane, e) order: everything of the lower lanes first
-                                uint32_t rr = cnt + __popc(bb[0] & lt_mask) + __popc(bb[1] & lt_mask) + __popc(bb[2] & lt_mask) + __popc(bb[3] & lt_mask);
-#pragma unroll
-                                for (int e = 0; e < 4; ++e) {
-                                    if (mt[e] && rr < (uint32_t)CAPW) s_q[idb + rr] = ((uint32_t)(s0 + e) << QSH) | jl[e];
-                                    rr += mt[e] ? 1u : 0u;
-                                }
-                                cnt += __popc(bb[0]) + __popc(bb[1]) + __popc(bb[2]) + __popc(bb[3]);
-                            }
-                        }
-                    } else {
-#pragma unroll
-                        for (int k = 0; k < KMAX; ++k) {
-                            if (k < K) {
-                                const int s = (warp * K + k) * 32 + lane;
-                                const uint32_t jl = jv[k] - (uint32_t)lo;
-                                const bool mt = (s < SC) && jl < (uint32_t)len;
-                                const uint32_t b = __ballot_sync(0xffffffffu, mt);
-                                const uint32_t rr = cnt + __popc(b & lt_mask);
-                                if (mt && rr < (uint32_t)CAPW) s_q[idb + rr] = ((uint32_t)s << QSH) | jl;
-                                cnt += __popc(b);
-                            }
-                        }
-                    }
-                    const bool ovf = cnt > (uint32_t)CAPW;
-                    if (ovf) cnt = CAPW;
-                    if (lane == 0) s_cnt[warp] = cnt;
-                    // the J values of the next chunk (the registers are free now)
-                    const int i_next = i_cur - SC;
-                    int K_next = 2, SC_next = 0;
-                    if (i_next >= i_min) {
-                        K_next = pick_k(i_next);
-                        SC_next = min(NT * K_next, i_next - i_min + 1);
-                        load_chunk(i_next, K_next, SC_next);
-                    }
-                    __syncwarp();
-                    // ---- S2: originals of the warp's slots (32 at a time), filter marks ----
-                    uint32_t q_[ITMAX];
-                    LT vt[ITMAX], vj[ITMAX];
-#pragma unroll
-                    for (int it = 0; it < ITMAX; ++it) {  // all loads first (the tops above the region come from global memory)
-                        q_[it] = 0xFFFFFFFFu;             // no slot
-                        vt[it] = (LT)0, vj[it] = (LT)0;
-                        const int rr = it * 32 + lane;
-                        if (rr < (int)cnt) {
-                            const uint32_t q = s_q[idb + rr];
-                            const uint32_t jl = q & ((1u << QSH) - 1u);
-                            const int i = i_cur - (int)(q >> QSH);
-                            q_[it] = q;
-                            vj[it] = s_slab[jl];
-                            vt[it] = (i < hi) ? s_slab[i - lo] : ld_cg<LT>(a0 + i);  // T(i): left there by the pass of i's own region
-                        }
-                    }
-#pragma unroll
-                    for (int it = 0; it < ITMAX; ++it) {
-                        if (q_[it] != 0xFFFFFFFFu) {
-                            const uint32_t jl = q_[it] & ((1u << QSH) - 1u);
-                            const int i = i_cur - (int)(q_[it] >> QSH);
-                            mark_pos(jl);
-                            if (i < hi) mark_pos((uint32_t)(i - lo));
-                            s_otop[idb + it * 32 + lane] = vt[it];
-                        }
-                    }
-                    SQB_CONVERGE();
-                    const int any_ovf = __syncthreads_or(ovf ? 1 : 0);
-                    uint32_t total = lane < NWARP ? s_cnt[lane] : 0u;
-#pragma unroll
-                    for (int d = 16; d >= 1; d >>= 1) total += __shfl_xor_sync(0xffffffffu, total, d);
-                    if (any_ovf || total > (uint32_t)HS) {
-                        // more matches than a warp segment or a window holds: forget the marks, scan half as many steps
-                        uint4* bz = reinterpret_cast<uint4*>(s_bits);
-                        for (int x = tid; x < NWB / 4; x += NT) bz[x] = make_uint4(0u, 0u, 0u, 0u);
-                        __syncthreads();
-                        K = max(2, K >> 1);
-                        SC = min(NT * K, i_cur - i_min + 1);
-                        load_chunk(i_cur, K, SC);
-                        continue;
-                    }
-                    // ---- S3: slots on multiply-marked positions: compacted per warp, registered in the tables ----
-                    uint32_t fastm = 0;  // bit it: this lane's slot of iteration it takes the plain swap
-                    uint32_t nslow = 0;
-#pragma unroll
-                    for (int it = 0; it < ITMAX; ++it) {
-                        if (it * 32 < (int)cnt) {
-                            bool fl = false;
-                            const bool ac = q_[it] != 0xFFFFFFFFu;
-                            if (ac) {
-                                const uint32_t jl = q_[it] & ((1u << QSH) - 1u);
-                                const int i = i_cur - (int)(q_[it] >> QSH);
-                                fl = marked_again(jl) || (i < hi && marked_again((uint32_t)(i - lo)));
-                            }
-                            const uint32_t fb = __ballot_sync(0xffffffffu, fl);
-                            if (fl) s_slow[warp * 32 + ((nslow + __popc(fb & lt_mask)) & 31u)] = (uint16_t)(idb + it * 32 + lane);
-                            nslow += __popc(fb);
-                            fastm |= ((ac && !fl) ? 1u : 0u) << it;
-                        }
-                    }
-                    // (more than 32 such slots in one warp: only tiny or adversarial segments; handled like an overflow)
-                    const bool sovf = nslow > 32u;
-                    __syncwarp();
-                    int sid = -1;
-                    uint32_t sjl = 0, slotT = 0, slotO = 0;
-                    int stop = 0;
-                    bool stfl = false, sofl = false, sself = false;
-                    LT svt = (LT)0, svj = (LT)0;
-                    if (!sovf && lane < (int)nslow) {
-                        sid = s_slow[warp * 32 + lane];
-                        const uint32_t q = s_q[sid];
-                        sjl = q & ((1u << QSH) - 1u);
-                        stop = i_cur - (int)(q >> QSH);
-                        const bool inreg = stop < hi;
-                        sself = inreg && (uint32_t)(stop - lo) == sjl;
-                        stfl = marked_again(sjl);
-                        sofl = inreg && marked_again((uint32_t)(stop - lo));
-                        svt = s_otop[sid];
-                        svj = s_slab[sjl];
-                        if (stfl && !sself) slotT = push_targeter(sjl, sid);
-                        if (sofl) slotO = insert_owner((uint32_t)(stop - lo), sid);
-                    }
-                    SQB_CONVERGE();
-                    const int any_sovf = __syncthreads_or(sovf ? 1 : 0);
-                    if (any_sovf) {
-                        // undo the registrations of the other warps, then retry with half the steps
-                        if (sid >= 0) {
-                            if (stfl && !sself) s_tabT[slotT] = SQB_EMPTY64;
-                            if (sofl) s_tabO[slotO] = SQB_EMPTY64;
-                        }
-                        uint4* bz = reinterpret_cast<uint4*>(s_bits);
-                        for (int x = tid; x < NWB / 4; x += NT) bz[x] = make_uint4(0u, 0u, 0u, 0u);
-                        __syncthreads();
-                        K = max(1, K >> 1);  // K = 1: at most 32 slots per warp
-                        SC = min(NT * K, i_cur - i_min + 1);
-                        load_chunk(i_cur, K, SC);
-                        continue;
-                    }
-                    // ---- S4: writes.  Plain swaps by the lanes that hold them, everything else by the warp's resolver lanes
-                    //      from the (now immutable) lists and original values ----
-                    {
-                        uint4* bz = reinterpret_cast<uint4*>(s_bits);  // nobody reads the filter any more
-#pragma unroll
-                        for (int x = tid; x < NWB / 4; x += NT) bz[x] = make_uint4(0u, 0u, 0u, 0u);
-                    }
-#pragma unroll
-                    for (int it = 0; it < ITMAX; ++it) {
-                        if ((fastm >> it) & 1u) {
-                            const uint32_t jl = q_[it] & ((1u << QSH) - 1u);
-                            const int i = i_cur - (int)(q_[it] >> QSH);
-                            s_slab[jl] = vt[it];
-                            if (i < hi) s_slab[i - lo] = vj[it];
-                            else st_cs<LT>(a0 + i, vj[it]);  // final
-                        }
-                    }
-                    if (sid >= 0) {
-                        // T(x): value of slot x's top just before step x
-                        auto T_of = [&](int x) -> LT {
-                            while (true) {
-                                const int ix = i_cur - (int)(s_q[x] >> QSH);
-                                if (ix >= hi) break;  // tops above the region are never targets
-                                const int h = find_key(s_tabT, (uint32_t)(ix - lo));
-                                if (h < 0) break;
-                                int mx = -1;
-                                for (uint32_t e = (uint32_t)s_tabT[h] & 0xFFFFu; e != SQB_NONE16; e = s_next[e]) mx = max(mx, (int)e);
-                                x = mx;  // the latest targeter of x's top (every targeter of a top precedes its step)
-                            }
-                            return s_otop[x];
-                        };
-                        const LT Ts = sofl ? T_of(sid) : svt;
-                        LT val = svj;
-                        if (sself) {
-                            val = Ts;
-                        } else {
-                            bool last = true;  // the only (or the last) slot of this window that targets the position
-                            if (stfl) {
-                                const uint32_t head = (uint32_t)s_tabT[slotT] & 0xFFFFu;
-                                int mx;
-                                const int p = sqb_list_latest_before(s_next, head, sid, &mx);
-                                if (p >= 0) val = T_of(p);
-                                last = (mx == sid);
-                            }
-                            if (last && !(stfl && find_key(s_tabO, sjl) >= 0)) s_slab[sjl] = Ts;
-                        }
-                        if (stop < hi) s_slab[stop - lo] = val;
-                        else st_cs<LT>(a0 + stop, val);  // final
-                    }
-                    SQB_CONVERGE();
-                    __syncthreads();
-                    // ---- S5: the resolver lanes clear their table entries (ordered before the next window's pushes by its
-                    //      first barrier; the filter was cleared above) ----
-                    if (sid >= 0) {
-                        if (stfl && !sself) s_tabT[slotT] = SQB_EMPTY64;
-                        if (sofl) s_tabO[slotO] = SQB_EMPTY64;
-                    }
-                    i_cur = i_next;
-                    K = K_next;
-                    SC = SC_next;
-                }
-                __syncthreads();
-                {  // a[lo, hi) <- slab
-                    LT* __restrict__ dst = a0 + lo;
-                    int x0 = 0;
-                    if ((reinterpret_cast<uintptr_t>(dst) & 15u) == 0) {
-                        constexpr int EPV = 16 / (int)sizeof(LT);
-                        const int nv = len / EPV;
-                        uint4* dv = reinterpret_cast<uint4*>(dst);
-                        const uint4* sv = reinterpret_cast<const uint4*>(s_slab);
-                        for (int x = tid; x < nv; x += NT) dv[x] = sv[x];
-                        x0 = nv * EPV;
-                    }
-                    for (int x = x0 + tid; x < len; x += NT) dst[x] = s_slab[x];
-                }
-                __syncthreads();
-            }
-        }
-    }
-}
-#endif  // SQB_TEST_VARIANTS
-
-// ------------------------------------------------------------------------------------------------
 // 3. transpose [P][stride] -> [PB/32][n + 1][32]  (32 permutations x 256 nodes per CTA), optional row scatter through
 //    `order` (library-grouped position k -> original node id)
 // ------------------------------------------------------------------------------------------------
@@ -2571,7 +1049,7 @@ __global__ void __launch_bounds__(256) nhood_transpose_kernel(const LT* __restri
 }
 
 // ------------------------------------------------------------------------------------------------
-// 2c. Fast RNG mode ("philox"): no replay of numpy's stream, no Fisher-Yates, no permutation-major label rows.
+// 2f. Fast RNG mode ("philox"): no replay of numpy's stream, no Fisher-Yates, no permutation-major label rows.
 //     Permutation p of a segment of m labels is a KEYED BIJECTION pi_p on [0, m): a generalised Feistel network
 //     (Black & Rogaway's FE2) on the mixed-radix domain [0, a) x [0, b), a = ceil(sqrt(m)), b = ceil(m / a), so that
 //     a*b - m < a and cycle walking (re-encrypt while the value is >= m) practically never happens (m = 10^6: 1 value
@@ -3162,12 +1640,11 @@ struct sqb_nhood {
     DevBuf<uint32_t> d_tmp_u32;
     std::vector<uint32_t> h_order;
     // options
-    int shuffle_algo = -1;  // -1 auto (1 for few permutations, else 2); 0 serial thread per permutation (cross-check);
-                            // 1 CTA per permutation; 2 warp per permutation; 3 CTA per permutation, large windows
-    int shuffle_q = 4;     // algo 2: PCG64 outputs per lane per batch (window = 64*q raw values)
-    int shuffle_r = 4;     // algo 3: PCG64 outputs per thread per batch (window = 2*r*threads raw values); algo 5: steps per thread
-    int64_t shuffle_low = 0;   // algo 5: elements of every label array kept in shared memory (-1 = as much as fits, 0 = off)
-    int64_t shuffle_region = 0;  // algo 8: positions per region (0 = as many as shared memory holds; smaller values are a test hook)
+    int shuffle_algo = -1;  // -1 auto (see launch_shuffle); 1 CTA per permutation (2a); 2 warp per permutation (2b);
+                            // 7 swap-target generation + list apply (2d, 2e)
+    int shuffle_q = 4;     // algos 2, 7: PCG64 outputs per lane per batch (window = 64*q raw values)
+    int shuffle_r = 4;     // algo 7: Fisher-Yates steps per thread and window (window = r*threads steps)
+    int64_t shuffle_low = 0;   // algo 7: elements of every label array kept in shared memory (-1 = as much as fits, 0 = off)
     int64_t shuffle_stagger_us = 0;  // start-up stagger of the persistent shuffle CTAs / warps (see sqb_stagger)
     int shuffle_threads = 512;
     int64_t perm_chunk = 0;  // 0 = auto
@@ -3287,81 +1764,6 @@ static int launch_shuffle_nt(sqb_nhood* h, LT* lab, const uint64_t* states, int6
     return SQB_OK;
 }
 
-#ifdef SQB_TEST_VARIANTS  // superseded replay variant: compiled into the test build only (tests/native/libsquidpy_b200_testvariants.so)
-template <typename LT, int NT, int R>
-static int launch_shuffle_cta2(sqb_nhood* h, LT* lab, const uint64_t* states, int64_t np) {
-    sqb_ctx* c = h->ctx;
-    auto k = nhood_shuffle_cta2_kernel<LT, NT, R>;
-    constexpr size_t RAW = (size_t)2 * R * NT, HS = 2 * RAW;
-    const size_t smem = HS * 8 + RAW * 4 + (RAW / 32) * 4 + (size_t)R * 32 * 4 + 16 + RAW * sizeof(LT) + HS * sizeof(LT);
-    SQB_CHECK(smem <= c->smem_optin, SQB_ERR_UNSUPPORTED, "shuffle_algo 3: %zu bytes of shared memory exceed the device limit", smem);
-    SQB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int64_t grid = h->shuffle_ctas;
-    if (grid <= 0) {
-        int per_sm = 1;
-        SQB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, NT, smem));
-        if (per_sm < 1) per_sm = 1;
-        grid = (int64_t)per_sm * c->sm_count;
-    }
-    if (grid > np) grid = np;
-    k<<<(unsigned)grid, NT, smem, c->stream>>>(lab, h->stride, states, np, h->nseg, h->d_seg_start.p, h->d_seg_len.p,
-                                               (float)h->shuffle_wfactor_x100 / 100.0f, 0xFFFFFFFFu,
-                                            (uint64_t)h->shuffle_stagger_us * 1000ull);
-    return SQB_OK;
-}
-
-template <typename LT, int NT, int R>
-static int launch_shuffle_list(sqb_nhood* h, LT* lab, const uint64_t* states, int64_t np) {
-    sqb_ctx* c = h->ctx;
-    auto k = nhood_shuffle_list_kernel<LT, NT, R>;
-    constexpr size_t RAW = (size_t)2 * R * NT, HS = 2 * RAW;
-    // [tab u64 x HS][ohead u32 x RAW][wsum int x 2*R*32][misc int x 4][next u16 x RAW][otop LT x RAW]
-    const size_t smem = HS * 8 + RAW * 4 + (size_t)2 * R * 32 * 4 + 16 + RAW * 2 + RAW * sizeof(LT);
-    SQB_CHECK(smem <= c->smem_optin, SQB_ERR_UNSUPPORTED, "shuffle_algo 6: %zu bytes of shared memory exceed the device limit", smem);
-    SQB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int64_t grid = h->shuffle_ctas;
-    if (grid <= 0) {
-        int per_sm = 1;
-        SQB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, NT, smem));
-        if (per_sm < 1) per_sm = 1;
-        grid = (int64_t)per_sm * c->sm_count;
-    }
-    if (grid > np) grid = np;
-    k<<<(unsigned)grid, NT, smem, c->stream>>>(lab, h->stride, states, np, h->nseg, h->d_seg_start.p, h->d_seg_len.p,
-                                               (float)h->shuffle_wfactor_x100 / 100.0f, 0xFFFFFFFFu,
-                                               (uint64_t)h->shuffle_stagger_us * 1000ull);
-    return SQB_OK;
-}
-
-template <typename LT, int NT, int SPT>
-static int launch_apply(sqb_nhood* h, LT* lab, const uint32_t* J, int64_t np, float wf) {
-    sqb_ctx* c = h->ctx;
-    auto k = nhood_apply_kernel<LT, NT, SPT>;
-    constexpr size_t W = (size_t)NT * SPT, HS = 2 * W;
-    const size_t tables = HS * 8 + W * 4 + (W / 32) * 4 + 16 + W * sizeof(LT) + HS * sizeof(LT);
-    SQB_CHECK(tables <= c->smem_optin, SQB_ERR_UNSUPPORTED, "shuffle_algo 5: %zu bytes of shared memory exceed the device limit", tables);
-    // shared-memory resident low part: everything the SM has left (one CTA per SM), unless switched off
-    int64_t low_cap = 0;
-    if (h->shuffle_low != 0) {
-        int64_t avail = ((int64_t)c->smem_optin - 1024 - (int64_t)tables) / (int64_t)sizeof(LT);
-        if (h->shuffle_low > 0 && avail > h->shuffle_low) avail = h->shuffle_low;
-        low_cap = avail > 0 ? (avail / 1024) * 1024 : 0;
-    }
-    const size_t smem = tables + (size_t)low_cap * sizeof(LT);
-    SQB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int64_t grid = h->shuffle_ctas;
-    if (grid <= 0) {
-        int per_sm = 1;
-        SQB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, NT, smem));
-        grid = (int64_t)(per_sm < 1 ? 1 : per_sm) * c->sm_count;
-    }
-    if (grid > np) grid = np;
-    k<<<(unsigned)grid, NT, smem, c->stream>>>(lab, J, h->stride, np, h->nseg, h->d_seg_start.p, h->d_seg_len.p, wf,
-                                               (int)low_cap, (uint64_t)h->shuffle_stagger_us * 1000ull);
-    return SQB_OK;
-}
-
-#endif  // SQB_TEST_VARIANTS
 template <typename LT, int NT, int SPT>
 static int launch_apply_list(sqb_nhood* h, LT* lab, const uint32_t* J, int64_t np, int64_t low) {
     sqb_ctx* c = h->ctx;
@@ -3391,44 +1793,11 @@ static int launch_apply_list(sqb_nhood* h, LT* lab, const uint32_t* J, int64_t n
     return SQB_OK;
 }
 
-#ifdef SQB_TEST_VARIANTS
-template <typename LT, int NT>
-static int launch_apply_region(sqb_nhood* h, LT* lab, const uint32_t* J, int64_t np) {
-    sqb_ctx* c = h->ctx;
-    auto k = nhood_apply_region_kernel<LT, NT>;
-    constexpr size_t NWARP = NT / 32, NID = NWARP * 96, HS = 2 * NT, NWB = 2 * HS;
-    // [tabT, tabO u64 x HS][bits u32 x NWB][q u32 x NID][cnt u32 x 64][next u16 x NID][slow u16 x 32 NWARP][otop LT x NID][slab LT x cap]
-    const size_t tables = 2 * HS * 8 + NWB * 4 + NID * 4 + 64 * 4 + NID * 2 + NWARP * 32 * 2 + NID * sizeof(LT);
-    SQB_CHECK(tables + 16 * sizeof(LT) <= c->smem_optin, SQB_ERR_UNSUPPORTED, "shuffle_algo 8: %zu bytes of shared memory exceed the device limit", tables);
-    int64_t cap = ((int64_t)c->smem_optin - (int64_t)tables) / (int64_t)sizeof(LT);
-    if (cap > (1 << 18) - 16) cap = (1 << 18) - 16;                                 // targets are stored in 18 bits (all ones = no slot)
-    if (h->shuffle_region > 0 && cap > h->shuffle_region) cap = h->shuffle_region;  // test hook: small regions
-    cap = (cap / 16) * 16;
-    if (cap < 16) cap = 16;
-    const size_t smem = tables + (size_t)cap * sizeof(LT);
-    SQB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int64_t grid = h->shuffle_ctas;
-    if (grid <= 0) grid = c->sm_count;  // one CTA per SM (launch bounds), persistent over the permutations
-    if (grid > np) grid = np;
-    k<<<(unsigned)grid, NT, smem, c->stream>>>(lab, J, h->stride, np, h->nseg, h->d_seg_start.p, h->d_seg_len.p, 0xFFFFFFFFu,
-                                               (uint64_t)h->shuffle_stagger_us * 1000ull, (int)cap);
-    return SQB_OK;
-}
-#endif  // SQB_TEST_VARIANTS
-
-#ifndef SQB_TEST_VARIANTS
-static int sqb_variant_unavailable(int algo) {
-    sqb_set_error("shuffle_algo %d is a superseded replay variant kept as a cross-check: it is compiled into the test build only "
-                  "(make -C squidpy_b200/csrc testvariants); the product library offers -1 (auto), 1, 2 and 7", algo);
-    return SQB_ERR_UNSUPPORTED;
-}
-#endif
-
+// shuffle_algo 7: swap-target generation (2d), then the list apply (2e) with nt threads, r steps per thread and window and
+// low elements of every label array in shared memory
 template <typename LT>
-static int launch_shuffle_two_kernel(sqb_nhood* h, LT* lab, const uint64_t* states, int64_t np, int algo, int nt, int r,
-                                     int64_t low) {
+static int launch_shuffle_two_kernel(sqb_nhood* h, LT* lab, const uint64_t* states, int64_t np, int nt, int r, int64_t low) {
     sqb_ctx* c = h->ctx;
-    const float wf = (float)h->shuffle_wfactor_x100 / 100.0f;
     SQB_TRY(c->scratch[2].alloc((size_t)np * h->stride * sizeof(uint32_t)));
     uint32_t* J = reinterpret_cast<uint32_t*>(c->scratch[2].p);
     {
@@ -3447,102 +1816,32 @@ static int launch_shuffle_two_kernel(sqb_nhood* h, LT* lab, const uint64_t* stat
     }
     SqbLaunchScope scope(c, SQB_K_NHOOD_SHUFFLE);
     int rc = SQB_ERR_INVALID;
-    if (algo == 8) {  // (shuffle_r is not used by this variant)
-#ifdef SQB_TEST_VARIANTS
-        if (nt == 1024) rc = launch_apply_region<LT, 1024>(h, lab, J, np);
-        else if (nt == 512) rc = launch_apply_region<LT, 512>(h, lab, J, np);
-        else if (nt == 256) rc = launch_apply_region<LT, 256>(h, lab, J, np);
-        else sqb_set_error("shuffle_algo 8: unsupported shuffle_threads = %d", nt);
-        SQB_TRY(rc);
-        SQB_POST_LAUNCH();
-        return SQB_OK;
-#else
-        return sqb_variant_unavailable(algo);
-#endif
-    }
-    if (algo == 7) {
-        if (nt == 1024 && r == 4) rc = launch_apply_list<LT, 1024, 4>(h, lab, J, np, low);
-        else if (nt == 1024 && r == 2) rc = launch_apply_list<LT, 1024, 2>(h, lab, J, np, low);
-        else if (nt == 512 && r == 8) rc = launch_apply_list<LT, 512, 8>(h, lab, J, np, low);
-        else if (nt == 512 && r == 4) rc = launch_apply_list<LT, 512, 4>(h, lab, J, np, low);
-        else if (nt == 512 && r == 2) rc = launch_apply_list<LT, 512, 2>(h, lab, J, np, low);
-        else if (nt == 256 && r == 8) rc = launch_apply_list<LT, 256, 8>(h, lab, J, np, low);
-        else if (nt == 256 && r == 4) rc = launch_apply_list<LT, 256, 4>(h, lab, J, np, low);
-        else if (nt == 128 && r == 4) rc = launch_apply_list<LT, 128, 4>(h, lab, J, np, low);
-        else sqb_set_error("shuffle_algo 7: unsupported (shuffle_threads, shuffle_r) = (%d, %d)", nt, r);
-        SQB_TRY(rc);
-        SQB_POST_LAUNCH();
-        return SQB_OK;
-    }
-#ifdef SQB_TEST_VARIANTS
-    if (nt == 512 && r == 4) rc = launch_apply<LT, 512, 4>(h, lab, J, np, wf);
-    else if (nt == 512 && r == 2) rc = launch_apply<LT, 512, 2>(h, lab, J, np, wf);
-    else if (nt == 1024 && r == 2) rc = launch_apply<LT, 1024, 2>(h, lab, J, np, wf);
-    else if (nt == 1024 && r == 4) rc = launch_apply<LT, 1024, 4>(h, lab, J, np, wf);
-    else if (nt == 256 && r == 4) rc = launch_apply<LT, 256, 4>(h, lab, J, np, wf);
-    else if (nt == 256 && r == 8) rc = launch_apply<LT, 256, 8>(h, lab, J, np, wf);
-    else sqb_set_error("shuffle_algo 5: unsupported (shuffle_threads, shuffle_r) = (%d, %d)", nt, r);
+    if (nt == 1024 && r == 4) rc = launch_apply_list<LT, 1024, 4>(h, lab, J, np, low);
+    else if (nt == 1024 && r == 2) rc = launch_apply_list<LT, 1024, 2>(h, lab, J, np, low);
+    else if (nt == 512 && r == 8) rc = launch_apply_list<LT, 512, 8>(h, lab, J, np, low);
+    else if (nt == 512 && r == 4) rc = launch_apply_list<LT, 512, 4>(h, lab, J, np, low);
+    else if (nt == 512 && r == 2) rc = launch_apply_list<LT, 512, 2>(h, lab, J, np, low);
+    else if (nt == 256 && r == 8) rc = launch_apply_list<LT, 256, 8>(h, lab, J, np, low);
+    else if (nt == 256 && r == 4) rc = launch_apply_list<LT, 256, 4>(h, lab, J, np, low);
+    else if (nt == 128 && r == 4) rc = launch_apply_list<LT, 128, 4>(h, lab, J, np, low);
+    else sqb_set_error("shuffle_algo 7: unsupported (shuffle_threads, shuffle_r) = (%d, %d)", nt, r);
     SQB_TRY(rc);
     SQB_POST_LAUNCH();
     return SQB_OK;
-#else
-    (void)wf;
-    (void)rc;
-    return sqb_variant_unavailable(algo);
-#endif
 }
 
 template <typename LT>
 static int launch_shuffle(sqb_nhood* h, LT* lab, const uint64_t* states, int64_t np) {
     sqb_ctx* c = h->ctx;
-    if (h->shuffle_algo == 5 || h->shuffle_algo == 7 || h->shuffle_algo == 8)
-        return launch_shuffle_two_kernel<LT>(h, lab, states, np, h->shuffle_algo, h->shuffle_threads, h->shuffle_r, h->shuffle_low);
+    if (h->shuffle_algo == 7) return launch_shuffle_two_kernel<LT>(h, lab, states, np, h->shuffle_threads, h->shuffle_r, h->shuffle_low);
     // auto (measured on B200, 1000 x 1M: two-kernel list replay 23 ms, warp per permutation 39 ms, CTA per permutation
     // 42 ms): many permutations of large arrays -> J generation + list apply with the tuned shape (1024 threads, 2048-step
     // windows, 96 K elements of every array in shared memory); few permutations -> one CTA each (finishes sooner);
     // many permutations of small arrays (L1/L2 resident) -> one warp each
     if (h->shuffle_algo < 0 && np > 2 * (int64_t)c->sm_count && h->n >= 65536)
-        return launch_shuffle_two_kernel<LT>(h, lab, states, np, 7, 1024, 2, 98304);
+        return launch_shuffle_two_kernel<LT>(h, lab, states, np, 1024, 2, 98304);
     SqbLaunchScope scope(c, SQB_K_NHOOD_SHUFFLE);
     const int algo = h->shuffle_algo >= 0 ? h->shuffle_algo : (np <= 2 * (int64_t)c->sm_count ? 1 : 2);
-#ifndef SQB_TEST_VARIANTS
-    if (algo == 0 || algo == 3 || algo == 4 || algo == 6) return sqb_variant_unavailable(algo);
-#else
-    if (algo == 0) {
-        nhood_shuffle_serial_kernel<LT><<<(unsigned)ceil_div64(np, 32), 32, 0, c->stream>>>(
-            lab, h->stride, states, np, h->nseg, h->d_seg_start.p, h->d_seg_len.p);
-    } else if (algo == 6) {
-        const int nt = (int)h->shuffle_threads, r = (int)h->shuffle_r;
-        int rc = SQB_ERR_UNSUPPORTED;
-        if (nt == 512 && r == 4) rc = launch_shuffle_list<LT, 512, 4>(h, lab, states, np);
-        else if (nt == 512 && r == 2) rc = launch_shuffle_list<LT, 512, 2>(h, lab, states, np);
-        else if (nt == 512 && r == 8) rc = launch_shuffle_list<LT, 512, 8>(h, lab, states, np);
-        else if (nt == 256 && r == 4) rc = launch_shuffle_list<LT, 256, 4>(h, lab, states, np);
-        else if (nt == 256 && r == 8) rc = launch_shuffle_list<LT, 256, 8>(h, lab, states, np);
-        else if (nt == 1024 && r == 2) rc = launch_shuffle_list<LT, 1024, 2>(h, lab, states, np);
-        else if (nt == 1024 && r == 4) rc = launch_shuffle_list<LT, 1024, 4>(h, lab, states, np);
-        else if (nt == 128 && r == 4) rc = launch_shuffle_list<LT, 128, 4>(h, lab, states, np);
-        else sqb_set_error("shuffle_algo 6: unsupported (shuffle_threads, shuffle_r) = (%d, %d)", nt, r);
-        SQB_TRY(rc);
-    } else if (algo == 3) {
-        int rc = SQB_ERR_INVALID;
-        const int nt = h->shuffle_threads, r = h->shuffle_r;
-        if (nt == 512 && r == 4) rc = launch_shuffle_cta2<LT, 512, 4>(h, lab, states, np);
-        else if (nt == 512 && r == 2) rc = launch_shuffle_cta2<LT, 512, 2>(h, lab, states, np);
-        else if (nt == 256 && r == 4) rc = launch_shuffle_cta2<LT, 256, 4>(h, lab, states, np);
-        else if (nt == 256 && r == 8) rc = launch_shuffle_cta2<LT, 256, 8>(h, lab, states, np);
-        else if (nt == 1024 && r == 2) rc = launch_shuffle_cta2<LT, 1024, 2>(h, lab, states, np);
-        else if (nt == 1024 && r == 4) rc = launch_shuffle_cta2<LT, 1024, 4>(h, lab, states, np);
-        else if (nt == 128 && r == 4) rc = launch_shuffle_cta2<LT, 128, 4>(h, lab, states, np);
-        else sqb_set_error("shuffle_algo 3: unsupported (shuffle_threads, shuffle_r) = (%d, %d)", nt, r);
-        SQB_TRY(rc);
-    } else if (algo == 4) {
-        int64_t ctas = h->shuffle_ctas > 0 ? h->shuffle_ctas : (int64_t)c->sm_count * 6;
-        if (ctas > ceil_div64(np, PIPE_TEAMS)) ctas = ceil_div64(np, PIPE_TEAMS);
-        nhood_shuffle_pipe_kernel<LT><<<(unsigned)ctas, PIPE_TEAMS * 64, 0, c->stream>>>(
-            lab, h->stride, states, np, h->nseg, h->d_seg_start.p, h->d_seg_len.p, (float)h->shuffle_wfactor_x100 / 100.0f);
-    } else
-#endif
     if (algo == 2) {
         const float wf = (float)h->shuffle_wfactor_x100 / 100.0f;
         int64_t ctas = h->shuffle_ctas > 0 ? h->shuffle_ctas : (int64_t)c->sm_count * 8;
@@ -3587,7 +1886,7 @@ static int launch_shuffle(sqb_nhood* h, LT* lab, const uint64_t* states, int64_t
 static int64_t auto_chunk(sqb_nhood* h) {
     if (h->perm_chunk > 0) return ((h->perm_chunk + 31) / 32) * 32;
     // keep [chunk][stride] + [n][chunk] under ~8 GB
-    int64_t per_perm = 2 * h->stride * h->lt_bytes + 4 * h->stride;  // label matrices + uint32 target lists (algo 5)
+    int64_t per_perm = 2 * h->stride * h->lt_bytes + 4 * h->stride;  // label matrices + uint32 target lists (algo 7)
     int64_t ch = (int64_t)8e9 / (per_perm > 0 ? per_perm : 1);
     if (ch < 32) ch = 32;
     if (ch > 16384) ch = 16384;
@@ -4027,7 +2326,7 @@ int sqb_nhood_destroy(sqb_nhood* h) {
 int sqb_nhood_set_option(sqb_nhood* h, const char* key, int64_t value) {
     SQB_CHECK(h && key, SQB_ERR_INVALID, "sqb_nhood_set_option: null argument");
     if (!strcmp(key, "shuffle_algo")) {
-        SQB_CHECK(value >= -1 && value <= 8, SQB_ERR_INVALID, "shuffle_algo must be -1 (auto) or 0..8");
+        SQB_CHECK(value == -1 || value == 1 || value == 2 || value == 7, SQB_ERR_INVALID, "shuffle_algo must be -1 (auto), 1, 2 or 7");
         h->shuffle_algo = (int)value;
     } else if (!strcmp(key, "jgen_threads")) {
         SQB_CHECK(value == 32 || value == 64 || value == 128, SQB_ERR_INVALID, "jgen_threads must be 32, 64 or 128");
@@ -4046,14 +2345,11 @@ int sqb_nhood_set_option(sqb_nhood* h, const char* key, int64_t value) {
     } else if (!strcmp(key, "shuffle_low")) {
         SQB_CHECK(value >= -1, SQB_ERR_INVALID, "shuffle_low must be >= -1");
         h->shuffle_low = value;
-    } else if (!strcmp(key, "shuffle_region")) {
-        SQB_CHECK(value >= 0, SQB_ERR_INVALID, "shuffle_region must be >= 0");
-        h->shuffle_region = value;
     } else if (!strcmp(key, "shuffle_r")) {
         SQB_CHECK(value == 2 || value == 4 || value == 8, SQB_ERR_INVALID, "shuffle_r must be 2, 4 or 8");
         h->shuffle_r = (int)value;
     } else if (!strcmp(key, "shuffle_q")) {
-        SQB_CHECK(value == 1 || value == 2 || value == 4 || value == 8, SQB_ERR_INVALID, "shuffle_q must be 1, 2, 4 or 8 (8: algos 5, 7 only)");
+        SQB_CHECK(value == 1 || value == 2 || value == 4 || value == 8, SQB_ERR_INVALID, "shuffle_q must be 1, 2, 4 or 8 (8: algo 7 only)");
         h->shuffle_q = (int)value;
     } else if (!strcmp(key, "shuffle_threads")) {
         SQB_CHECK(value == 128 || value == 256 || value == 512 || value == 1024, SQB_ERR_INVALID,

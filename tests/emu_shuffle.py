@@ -4,7 +4,7 @@ It mirrors the device algorithm phase by phase (RNG batch by jump-ahead, windowe
 hash-based conflict detection, parallel swaps + ordered serial pass) so the *algorithm* can be validated on
 the CPU against numpy's ``Generator.shuffle`` (tests/test_shuffle_emulation.py).  Not used by the product.
 
-Also here: ``resolve_window_lists`` (the serial-pass-free conflict resolution of shuffle_algo 6 / 7) and ``emu_targets``
+Also here: ``resolve_window_lists`` (the serial-pass-free conflict resolution of shuffle_algo 7) and ``emu_targets``
 (nhood_jgen_kernel: batch-sized windows, one-pass acceptance), each the executable specification of its kernel.
 """
 from __future__ import annotations
@@ -43,7 +43,7 @@ def window_size(i_cur, raw_left, raw_total):
 
 
 def resolve_window_lists(a, base, i_cur, sj, rng):
-    """Conflict resolution WITHOUT a serial pass (shuffle_algo 6, nhood_shuffle_list_kernel): applies the window's steps
+    """Conflict resolution WITHOUT a serial pass (shuffle_algo 7, nhood_apply_list_kernel): applies the window's steps
     s = 0..S-1 (swap positions i_cur-s and sj[s]) to `a` in place.  Every step pushes itself on the list of the position
     it targets (arbitrary push order = thread interleaving); afterwards each step derives what it has to write from the
     lists alone, reading only ORIGINAL values:
@@ -325,7 +325,7 @@ def serial_targets(state, inc, segs):
 
 
 # ------------------------------------------------------------------------------------------------
-# Region replay (shuffle_algo 8, nhood_apply_region_kernel): executable specification
+# Region replay: executable specification of nhood_apply_region_kernel (shuffle_algo 8, last present in commit eef2f18)
 # ------------------------------------------------------------------------------------------------
 def _resolve_general_window(slab, a, lo, hi, tops, tgts, rng):
     """One window of the region replay: compacted steps in step order (slot s: top position tops[s], strictly descending;
@@ -376,7 +376,7 @@ def _resolve_general_window(slab, a, lo, hi, tops, tgts, rng):
 
 def region_replay(arr, J, cap, NT=8, WL=4, CAPW=12, KMAX=16, rng=None, stats=None):
     """Applies the Fisher-Yates steps i = m-1 .. 1 (swap positions i and J[i] <= i) to a copy of `arr`, one region of at most
-    `cap` positions at a time, top region first (see nhood.cu 2i): the pass of region [lo, hi) scans all steps i >= lo and
+    `cap` positions at a time, top region first (see DESIGN.md 3.1): the pass of region [lo, hi) scans all steps i >= lo and
     applies those whose TARGET lies in the region (a step whose target lies below is left to a later pass: its top then
     still holds T(step), the value it had just before the step).  Mirrors the kernel's chunking: NT*K steps are scanned per
     window, "warp" w (WL lanes) takes the w-th run of WL*K of them; K is sized for ~0.58 CAPW expected matches per warp and

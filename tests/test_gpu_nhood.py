@@ -2,10 +2,6 @@
 
 from __future__ import annotations
 
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pandas as pd
 import pytest
@@ -18,18 +14,6 @@ from squidpy_b200.gr import NhoodPlan
 from tools import synth
 
 pytestmark = pytest.mark.gpu
-
-# The product library offers the replay variants -1 (auto), 1, 2 and 7.  The superseded variants 0, 3, 4, 5, 6 and the slower region replay 8 are kept as
-# independent cross-checks in a TEST build of the same sources (tests/native/libsquidpy_b200_testvariants.so, `make testvariants`):
-# `test_superseded_replay_variants_cross_check` re-runs this file against that build in a subprocess with SQB_VARIANT_TESTS=1,
-# which flips the parametrisations below from the product variants to the superseded ones.
-VARIANT_RUN = os.environ.get("SQB_VARIANT_TESTS") == "1"
-PRODUCT_ALGOS = (-1, 1, 2, 7)
-
-
-def _algos(params):
-    return [q for q in params if ((q[0] if isinstance(q, tuple) else q) in PRODUCT_ALGOS) != VARIANT_RUN]
-
 
 
 def _plan(g, n_cls):
@@ -139,25 +123,19 @@ def test_create_errors():
         NhoodPlan(np.array([0, 1, 2]), np.array([1, -1], dtype=np.int64), 2)
 
 
-@pytest.mark.parametrize("algo,threads,q", _algos([(0, 512, 4), (1, 128, 4), (1, 256, 4), (1, 512, 4), (1, 1024, 4), (2, 512, 1), (2, 512, 2), (2, 512, 4),
-                                             (3, 128, 4), (3, 256, 4), (3, 256, 8), (3, 512, 2), (3, 512, 4), (3, 1024, 2), (3, 1024, 4), (4, 512, 4),
-                                             (5, 256, 4), (5, 256, 8), (5, 512, 2), (5, 512, 4), (5, 1024, 2), (5, 1024, 4),
-                                             (6, 128, 4), (6, 256, 4), (6, 256, 8), (6, 512, 2), (6, 512, 4), (6, 512, 8), (6, 1024, 2), (6, 1024, 4),
-                                             (7, 128, 4), (7, 256, 4), (7, 256, 8), (7, 512, 2), (7, 512, 4), (7, 512, 8), (7, 1024, 2), (7, 1024, 4),
-                                             (8, 256, 4), (8, 512, 2), (8, 512, 4), (8, 1024, 2)]))
+@pytest.mark.parametrize("algo,threads,q", [(1, 128, 4), (1, 256, 4), (1, 512, 4), (1, 1024, 4), (2, 512, 1), (2, 512, 2), (2, 512, 4),
+                                             (7, 128, 4), (7, 256, 4), (7, 256, 8), (7, 512, 2), (7, 512, 4), (7, 512, 8), (7, 1024, 2), (7, 1024, 4)])
 @pytest.mark.parametrize("n", [2, 3, 5, 33, 100, 1000, 1025, 5041, 70001])
 def test_shuffle_is_numpy_exact(algo, threads, q, n):
     """Shuffled label vectors equal numpy Generator.shuffle of the same spawned generators (oracle = exact replay,
     pinned to numpy in tests/test_oracle_golden.py)."""
-    if algo == 0 and n > 6000:
-        pytest.skip("serial cross-check kernel: small sizes only")
     g = sp.csr_matrix((np.ones(n - 1, np.float32), (np.arange(n - 1), np.arange(1, n))), shape=(n, n))
     n_cls = 251
     base = (np.arange(n) % n_cls).astype(np.uint32)
     plan = _plan(g, n_cls)
     plan.set_option("shuffle_algo", algo)
     plan.set_option("shuffle_threads", threads)
-    plan.set_option("shuffle_r" if algo in (3, 5, 6, 7, 8) else "shuffle_q", q)
+    plan.set_option("shuffle_r" if algo == 7 else "shuffle_q", q)
     plan.set_base(base)
     P = 7
     st = spawn_states(1234 + n, P)
@@ -166,7 +144,7 @@ def test_shuffle_is_numpy_exact(algo, threads, q, n):
     np.testing.assert_array_equal(got, ref.shuffle_labels(base, st))
 
 
-@pytest.mark.parametrize("algo,threads,r", _algos([(1, 512, 4), (2, 512, 4), (3, 512, 4), (5, 512, 4), (6, 512, 4), (6, 1024, 2), (7, 1024, 2), (7, 512, 8), (8, 1024, 2), (8, 512, 4), (-1, 512, 4)]))
+@pytest.mark.parametrize("algo,threads,r", [(1, 512, 4), (2, 512, 4), (7, 1024, 2), (7, 512, 8), (-1, 512, 4)])
 def test_shuffle_uint16_labels(algo, threads, r):
     """More than 256 categories: 16-bit label arrays through every replay variant (incl. the shared-memory low part of the
     default, which then holds half as many elements), with library segments."""
@@ -178,11 +156,9 @@ def test_shuffle_uint16_labels(algo, threads, r):
     plan = _plan(g, n_cls)
     plan.set_option("shuffle_algo", algo)
     plan.set_option("shuffle_threads", threads)
-    plan.set_option("shuffle_r" if algo in (3, 5, 6, 7, 8) else "shuffle_q", r)
+    plan.set_option("shuffle_r" if algo == 7 else "shuffle_q", r)
     if algo == 7:
         plan.set_option("shuffle_low", -1)
-    if algo == 8:
-        plan.set_option("shuffle_region", 20000)  # several regions per segment
     P = 300 if algo == -1 else 5  # auto picks the two-kernel list replay only for more than 2 x SM permutations
     st = spawn_states(11, P)
     plan.set_base(base)
@@ -196,77 +172,24 @@ def test_shuffle_uint16_labels(algo, threads, r):
 @pytest.mark.parametrize("q", [2, 4, 8])
 @pytest.mark.parametrize("n", [9, 257, 1000, 4099, 70001])
 def test_target_generation_batch_sizes(q, n):
-    """Swap-target generation of the two-kernel replays (128 / 256 raw values per batch).  Small arrays are the hard case for
+    """Swap-target generation of the two-kernel replay (128 / 256 raw values per batch).  Small arrays are the hard case for
     its acceptance fixed point: a window covers a quarter of the remaining range, so many candidates depend on their rank."""
     g = sp.csr_matrix((np.ones(n - 1, np.float32), (np.arange(n - 1), np.arange(1, n))), shape=(n, n))
     base = (np.arange(n) % 113).astype(np.uint32)
     st = spawn_states(900 + n, 24)
     exp = ref.shuffle_labels(base, st)
-    for algo in _algos([5, 7, 8]):
-        plan = _plan(g, 113)
-        plan.set_option("shuffle_algo", algo)
-        plan.set_option("shuffle_q", q)
-        plan.set_base(base)
-        plan.upload(st)
-        np.testing.assert_array_equal(plan.shuffled_labels(0, 24), exp)
-
-
-@pytest.mark.skipif(not VARIANT_RUN, reason="algo 6 lives in the test build (see test_superseded_replay_variants_cross_check)")
-@pytest.mark.parametrize("wf", [100, 400, 1600, 6400])
-@pytest.mark.parametrize("threads,r", [(256, 4), (512, 8), (1024, 4)])
-def test_list_replay_window_factor(wf, threads, r):
-    """algo 6 resolves conflicting swaps from per-position lists instead of an ordered pass; large window factors make
-    conflicts (and chains of conflicts) frequent.  Any window size must give numpy's permutation."""
-    n = 30011
-    g = sp.csr_matrix((np.ones(n - 1, np.float32), (np.arange(n - 1), np.arange(1, n))), shape=(n, n))
-    base = (np.arange(n) % 199).astype(np.uint32)
-    plan = _plan(g, 199)
-    plan.set_option("shuffle_algo", 6)
-    plan.set_option("shuffle_threads", threads)
-    plan.set_option("shuffle_r", r)
-    plan.set_option("shuffle_wfactor_x100", wf)
+    plan = _plan(g, 113)
+    plan.set_option("shuffle_algo", 7)
+    plan.set_option("shuffle_q", q)
     plan.set_base(base)
-    st = spawn_states(4321 + wf, 9)
     plan.upload(st)
-    np.testing.assert_array_equal(plan.shuffled_labels(0, 9), ref.shuffle_labels(base, st))
+    np.testing.assert_array_equal(plan.shuffled_labels(0, 24), exp)
 
 
-@pytest.mark.skipif(not VARIANT_RUN, reason="algo 8 lives in the test build (see test_superseded_replay_variants_cross_check)")
-@pytest.mark.parametrize("region", [16, 48, 1000, 4096, 30000, 65536, 0])
-@pytest.mark.parametrize("threads,r", [(1024, 2), (256, 4)])
-def test_region_replay_region_sizes(region, threads, r):
-    """algo 8 replays one region of the label array at a time in shared memory (tops above the region: compacted windows;
-    tops inside: consecutive windows; targets below: deferred to the pass that owns them).  Any region size must give numpy's
-    permutation: tiny regions make every step cross regions and the compaction windows sparse, region sizes around the window
-    length exercise the own-range lists next to deferred steps, 0 = everything shared memory holds."""
-    if region in (16, 48):
-        ns = [2, 17, 100, 3001]
-    else:
-        ns = [5041, 70001, 200003]
-    for n in ns:
-        g = sp.csr_matrix((np.ones(n - 1, np.float32), (np.arange(n - 1), np.arange(1, n))), shape=(n, n))
-        base = (np.arange(n) * 13 % 241).astype(np.uint32)
-        plan = _plan(g, 241)
-        plan.set_option("shuffle_algo", 8)
-        plan.set_option("shuffle_threads", threads)
-        plan.set_option("shuffle_r", r)
-        plan.set_option("shuffle_region", region)
-        plan.set_base(base)
-        st = spawn_states(555 + n + region, 4)
-        plan.upload(st)
-        np.testing.assert_array_equal(plan.shuffled_labels(0, 4), ref.shuffle_labels(base, st))
-        if n > 5000:
-            lib = (np.arange(n) % 3).astype(np.int32)
-            plan.set_base(base, lib, 3)
-            plan.upload(st)
-            np.testing.assert_array_equal(plan.shuffled_labels(0, 2), ref.shuffle_labels(base, st[:2], lib, 3))
-        plan.close()
-
-
-@pytest.mark.parametrize("algo", _algos([5, 7]))
+@pytest.mark.parametrize("algo", [7])
 @pytest.mark.parametrize("low", [0, 1024, 50000, -1])
 def test_two_kernel_replay_low_part(low, algo):
-    """algos 5 and 7 can keep the first `low` positions of every label array in shared memory: same permutations for any split."""
+    """algo 7 can keep the first `low` positions of every label array in shared memory: same permutations for any split."""
     n = 70001
     g = sp.csr_matrix((np.ones(n - 1, np.float32), (np.arange(n - 1), np.arange(1, n))), shape=(n, n))
     base = (np.arange(n) % 97).astype(np.uint32)
@@ -283,7 +206,7 @@ def test_two_kernel_replay_low_part(low, algo):
     np.testing.assert_array_equal(plan.shuffled_labels(0, 5), ref.shuffle_labels(base, st, lib, 3))
 
 
-@pytest.mark.parametrize("algo", _algos([0, 1, 2, 3, 4, 5, 6, 7, 8]))
+@pytest.mark.parametrize("algo", [1, 2, 7])
 def test_shuffle_library_groups(algo):
     n = 4000
     g = synth.hex_graph(40, 100)
@@ -424,8 +347,8 @@ def test_full_size_1m_spots():
     np.testing.assert_array_equal(got[:6], ref.nhood_perm_counts(g.indptr, g.indices, base, 30, st[:6]))
     assert (got.reshape(P, -1).sum(axis=1, dtype=np.int64) == g.nnz).all()  # every stored entry counted once
     np.testing.assert_array_equal(got, got.transpose(0, 2, 1))  # symmetric graph -> symmetric counts
-    # every replay variant at full size, incl. several permutations per CTA / team (the superseded ones in the test build)
-    for algo in ((3, 4, 5, 6, 8) if VARIANT_RUN else (1, 2, 7)):
+    # every replay at full size, incl. several permutations per CTA
+    for algo in (1, 2, 7):
         plan.set_option("shuffle_algo", algo)
         plan.set_option("shuffle_ctas", 16)
         np.testing.assert_array_equal(plan.permute(st), got)
@@ -451,35 +374,17 @@ def test_buffered_generator_states_are_rejected():
     plan.close()
 
 
-@pytest.mark.skipif(VARIANT_RUN, reason="already inside the cross-check run")
-def test_superseded_replay_variants_cross_check():
-    """The five superseded exact-replay variants (serial, large-window CTA, two-warp pipeline, ordered two-kernel, fused list
-    kernel) must produce numpy's permutations too: independent implementations of the same replay agreeing bit for bit is the
-    strongest check the product kernels have.  They are compiled into a test-only build, loaded here in a subprocess."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    lib = os.path.join(root, "tests", "native", "libsquidpy_b200_testvariants.so")
-    assert os.path.exists(lib), "build it with `make -C squidpy_b200/csrc testvariants` (done by __graft_entry__.build())"
-    env = dict(os.environ, SQB_LIB_PATH=lib, SQB_VARIANT_TESTS="1")
-    sel = "shuffle_is_numpy_exact or uint16_labels or target_generation or list_replay or low_part or library_groups or full_size_1m or region_replay"
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-m", "gpu", "-p", "no:cacheprovider", "-x", "-k", sel],
-                       env=env, capture_output=True, text=True, timeout=1700, cwd=root)
-    tail = (r.stdout + r.stderr)[-3000:]
-    assert r.returncode == 0, tail
-    import re
-
-    m = re.search(r"(\d+) passed", r.stdout)
-    assert m and int(m.group(1)) >= 250, tail
-
-
-def test_product_library_rejects_superseded_variants():
-    if VARIANT_RUN:
-        pytest.skip("test build")
+def test_set_option_rejects_unknown_replays():
+    """shuffle_algo takes -1 (auto), 1, 2 and 7; anything else is refused when it is set, and the plan keeps working."""
     g = synth.hex_graph(12, 12)
+    base = np.random.default_rng(0).integers(0, 4, g.shape[0]).astype(np.uint32)
     plan = _plan(g, 4)
-    plan.set_base(np.random.default_rng(0).integers(0, 4, g.shape[0]).astype(np.uint32))
-    for algo in (0, 3, 4, 5, 6, 8):
-        plan.set_option("shuffle_algo", algo)
-        with pytest.raises(NotImplementedError, match="test build"):
-            plan.permute(spawn_states(1, 3))
+    plan.set_base(base)
+    for algo in (-2, 0, 3, 4, 5, 6, 8, 9):
+        with pytest.raises(ValueError, match="shuffle_algo must be"):
+            plan.set_option("shuffle_algo", algo)
+    with pytest.raises(ValueError, match="unknown key 'shuffle_region'"):
+        plan.set_option("shuffle_region", 0)
     plan.set_option("shuffle_algo", -1)
-    assert plan.permute(spawn_states(1, 3)).shape == (3, 4, 4)
+    st = spawn_states(1, 3)
+    np.testing.assert_array_equal(plan.permute(st), ref.nhood_perm_counts(g.indptr, g.indices, base, 4, st))

@@ -47,7 +47,7 @@ def test_emulated_cta_shuffle_segments():
 
 
 def test_list_resolution_equals_serial_swaps():
-    """The serial-pass-free conflict resolution of shuffle_algo 6 (tests/emu_shuffle.resolve_window_lists) against the
+    """The serial-pass-free conflict resolution of shuffle_algo 7 (tests/emu_shuffle.resolve_window_lists) against the
     plain in-order application of the same swaps, on windows far denser in conflicts than the device ever sees."""
     from tests.emu_shuffle import resolve_window_lists
 
@@ -146,11 +146,11 @@ def _fisher_yates(arr, J):
 
 
 def test_region_replay_equals_fisher_yates():
-    """shuffle_algo 8 (tests/emu_shuffle.region_replay = the specification of nhood_apply_region_kernel): applying every step in
-    the pass of the region its TARGET falls into -- tops above the region through compacted windows, tops inside through
-    consecutive windows, targets below deferred with T(step) left at the top -- equals the plain Fisher-Yates sweep, for any
-    region size, window size and target distribution (uniform like the real stream, and adversarial: many duplicates, many
-    own-range targets, all targets in one region)."""
+    """The region replay (tests/emu_shuffle.region_replay = the specification of nhood_apply_region_kernel, last present in
+    commit eef2f18): applying every step in the pass of the region its TARGET falls into -- tops above the region through
+    compacted windows, tops inside through consecutive windows, targets below deferred with T(step) left at the top -- equals
+    the plain Fisher-Yates sweep, for any region size, window size and target distribution (uniform like the real stream, and
+    adversarial: many duplicates, many own-range targets, all targets in one region)."""
     from tests.emu_shuffle import region_replay
 
     rnd = random.Random(5)

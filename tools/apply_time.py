@@ -11,7 +11,7 @@ from squidpy_b200.gr import NhoodPlan  # noqa: E402
 from tools import synth  # noqa: E402
 
 P = int(sys.argv[1]) if len(sys.argv) > 1 else 1000
-variants = sys.argv[2:] or ["-1:1024:2", "8:1024:2"]
+variants = sys.argv[2:] or ["-1:1024:2", "7:1024:4"]
 ctx = sq.default_context(0)
 g = synth.hex_graph(1000, 1000)
 base = synth.categorical_labels(g.shape[0], 30, seed=0).cat.codes.to_numpy().astype(np.uint32)

@@ -18,7 +18,7 @@ for st in $STAGES; do
     sanitizer)
       timeout 900 compute-sanitizer --tool memcheck --error-exitcode 7 python __graft_entry__.py smoke > $OUT/sanitizer_memcheck.log 2>&1; echo "memcheck smoke rc=$?" | tee -a $OUT/summary.txt
       # block barriers after divergent code fault on sm_100a when a warp arrives un-converged: synccheck the replay kernels
-      timeout 700 compute-sanitizer --tool synccheck --error-exitcode 7 python -m pytest tests/test_gpu_nhood.py -q -p no:cacheprovider -x -k "(shuffle_is_numpy_exact and (7-1024-2 or 6-1024-2) and (70001 or 1025)) or (library_groups and (6 or 7)) or (uint16 and 7-1024)" > $OUT/sanitizer_synccheck.log 2>&1; echo "synccheck rc=$?" | tee -a $OUT/summary.txt
+      timeout 700 compute-sanitizer --tool synccheck --error-exitcode 7 python -m pytest tests/test_gpu_nhood.py -q -p no:cacheprovider -x -k "(shuffle_is_numpy_exact and 7-1024-2 and (70001 or 1025)) or (library_groups and 7) or (uint16 and 7-1024)" > $OUT/sanitizer_synccheck.log 2>&1; echo "synccheck rc=$?" | tee -a $OUT/summary.txt
       timeout 500 compute-sanitizer --tool memcheck --error-exitcode 7 python -m pytest tests/test_gpu_nhood.py -q -p no:cacheprovider -x -k "(shuffle_is_numpy_exact and 7-1024-2 and (70001 or 33)) or (library_groups and 7) or count_symmetric" > $OUT/sanitizer_memcheck2.log 2>&1; echo "memcheck nhood rc=$?" | tee -a $OUT/summary.txt
       tail -n 3 $OUT/sanitizer_memcheck.log $OUT/sanitizer_synccheck.log $OUT/sanitizer_memcheck2.log ;;
     bench)

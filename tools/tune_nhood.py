@@ -44,9 +44,6 @@ def main():
     variants.append({**a7, "shuffle_low": 65536, "shuffle_q": 8})
     variants.append({**a7, "shuffle_low": 65536, "shuffle_q": 2})
     variants.append({**a7, "shuffle_r": 4, "shuffle_low": 0})
-    if os.environ.get("SQB_LIB_PATH", "").endswith("testvariants.so"):  # superseded variants exist in the test build only
-        variants.append({**base, "shuffle_algo": 6, "shuffle_threads": 1024, "shuffle_r": 2, "shuffle_wfactor_x100": 1600})
-        variants.append({**base, "shuffle_algo": 5, "shuffle_threads": 512, "shuffle_r": 2})
     variants.append({**base, "shuffle_algo": 2})
     variants.append({**base, "shuffle_algo": 1, "shuffle_threads": 1024, "shuffle_ctas": 148})
     variants.append({**base, "shuffle_algo": -1, "count_sym": 0})
